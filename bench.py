@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's sm_100a path
   python bench.py --impl reference [--gpus N] [--steps K] ...    # the UNMODIFIED reference on the host cores
+  python bench.py ... --dump-outputs DIR                         # also save the last timed step's outputs as .npy
 
 Own arm.  A step is one pass of the training hot path over one synthetic batch: forward, BCE loss (+ confusion
 counts), backward, (N > 1: bucketed gradient all-reduce overlapped with the backward) and the Adam update of
@@ -36,6 +37,7 @@ if ROOT not in sys.path:
 TRAIN_GFLOP_PER_IMG_256 = 323.6      # SURVEY.md §2.2 / BASELINE.md: fwd + dgrad + wgrad conv FLOPs per image at 256x256
 FWD_GFLOP_PER_IMG_256 = 107.9
 REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+DUMP_MAX_ELEMS = 1 << 22     # per --dump-outputs array (16 MiB in float32): at most three arrays of this size per workload
 
 
 def load_peaks():
@@ -182,6 +184,8 @@ class Case:
         self.stage = [(torch.empty_like(self.x_dev), torch.empty_like(self.y_dev)) for _ in range(2)]
         self.copy_stream = torch.cuda.Stream(device=dev)
         self.staged = {"i": 0, "ev": None}
+        self.keep_last = False     # --dump-outputs: step() keeps its network output and result for outputs()
+        self.last = self.dumped = None
 
     # -- one step on device-resident inputs
     def step(self, x=None, y=None):
@@ -192,11 +196,17 @@ class Case:
         if self.kind == "infer":
             with torch.no_grad():
                 p = self.net(x)
-                return rbunet.confusion_counts(p, y)
+                counts = rbunet.confusion_counts(p, y)
+            if self.keep_last:
+                self.last = (p, counts)
+            return counts
         self.opt.zero_grad(set_to_none=True)
         if self.accum == 1:
-            loss = self.crit(self.net(x), y)
+            p = self.net(x)
+            loss = self.crit(p, y)
             loss.backward()
+            if self.keep_last:
+                self.last = (p, loss)
         else:
             mb = self.B // self.accum
             loss = None
@@ -230,6 +240,38 @@ class Case:
         st["cur"] = self._stage_next()                               # next step's inputs, behind this step's compute
         out = self.step(xs, ys)
         return out.cpu() if self.kind == "infer" else out.item()
+
+    def outputs(self):
+        """{name: float32/float64 numpy array} of what the last step() computed: the network output, the loss and
+        confusion counts and, for training, the gradients, the updated parameters and the BatchNorm running statistics.
+        An array above DUMP_MAX_ELEMS elements is reduced to a fixed seeded sample of its flattened values (the same
+        positions in every run of the same workload)."""
+        import numpy as np
+        import torch
+        torch.cuda.synchronize(self.env.dev)
+        p, res = self.last
+
+        def host(t):
+            t = t.detach()
+            if t.numel() > DUMP_MAX_ELEMS:
+                idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+                t = t.flatten()[torch.from_numpy(idx).to(t.device)]
+            t = t.double() if t.dtype in (torch.int64, torch.float64) else t.float()    # integers exact in float64
+            return t.cpu().numpy()
+
+        out = {"logits" if self.kind == "unet" else "probs": host(p)}
+        if self.kind == "infer":
+            out["confusion_counts"] = host(res)
+            return out
+        out["loss"] = host(res)
+        out["confusion_counts"] = host(self.crit.last_counts)
+        params = [q for q in self.model.parameters() if q.grad is not None]
+        out["grads"] = host(torch.cat([q.grad.flatten() for q in params]))
+        out["params"] = host(torch.cat([q.detach().flatten() for q in params]))
+        stats = [b.flatten() for n, b in self.model.named_buffers() if n.endswith(("running_mean", "running_var"))]
+        if stats:
+            out["bn_running_stats"] = host(torch.cat(stats))
+        return out
 
     def io_bytes(self):
         h2d = self.x_pin.numel() * 4 + self.y_pin.numel() * self.y_pin.element_size()
@@ -271,6 +313,9 @@ class Case:
     def measure(self, steps, warmup, e2e=True):
         """{value, ms_per_step, e2e, ...} of this case (images/s over all ranks, max-over-ranks device time)."""
         ms, launches, clocks, per = self.timed(self.step, steps, warmup)
+        if self.keep_last:
+            self.dumped = self.outputs()         # before the e2e steps below train the model further
+            self.keep_last, self.last = False, None
         imgs = self.B * self.env.world * steps
         rec = {"value": round(imgs / (ms / 1e3), 2), "unit": "img/s", "ms_per_step": round(ms / steps, 3), "steps": steps,
                "warmup": warmup, "gpu_launches": int(launches), "clocks": clocks, "ms_each_step": per}
@@ -393,6 +438,15 @@ def run_extra(env, name, kind, nc, S, B, steps, warmup, w_dice=0.0, accum=1, sca
     return rec
 
 
+def write_outputs(path, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array of Case.outputs()."""
+    import numpy as np
+    assert sum(a.nbytes for a in arrays.values()) <= 64 * 10 ** 6, {k: a.nbytes for k, a in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -408,7 +462,9 @@ def run_ours(args):
 
     torch.cuda.reset_peak_memory_stats(dev)
     case = Case(env, kind, nc, S, B, w_dice=args.w_dice)
+    case.keep_last = bool(args.dump_outputs)
     main = case.measure(args.steps, args.warmup)
+    dumped = case.dumped
     mem_per_px = torch.cuda.max_memory_allocated(dev) / (B * S * S)        # bytes per input pixel of the per-GPU batch
     # host time to ENQUEUE one step (no synchronisation inside): how close the launching thread is to being the bottleneck
     torch.cuda.synchronize()
@@ -473,6 +529,8 @@ def run_ours(args):
         out["extra"] = extra
 
     if rank == 0:
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         if world == 1 and not args.no_cpu_baseline and not unet:
             out["cpu_baseline"] = cpu_reference(infer, nc, S, budget_s=20.0)
         if world == 1 and not args.no_eager_baseline and kind == "train":
@@ -694,7 +752,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra.c3 / extra.c5 / extra.c4_infer sub-records")
     ap.add_argument("--no-flush", action="store_true", help="skip the 256 MiB L2-flush write between timed steps")
     ap.add_argument("--detail", default="", help="write the per-call device times of one profiled step to this file")
+    ap.add_argument("--dump-outputs", default="", dest="dump_outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32/float64, a fixed seeded "
+                         "sample of arrays above 4 Mi elements): outputs of two builds compare one to one")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs saves the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

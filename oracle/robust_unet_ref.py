@@ -7,9 +7,8 @@ product: only `tests/`, `__graft_entry__.smoke()` and `bench.py`'s cpu_baseline 
 
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md §4), so this
 restatement is pinned against outputs of the reference itself run in the build container
-(`oracle/make_golden.py` → `tests/golden/*.npz`, checked by `tests/test_oracle_golden.py`)
-and, when `/root/reference` is present, directly against `Main_Final.RobustUNet`
-(`tests/test_oracle_vs_reference.py`).  The RGB→HSV and Dice pieces have no reference code
+(`oracle/make_golden.py` → `tests/golden/*.npz`, checked by `tests/test_oracle_golden.py`).
+The RGB→HSV and Dice pieces have no reference code
 (SURVEY.md §8c): those two are "parity unpinned" — HSV is pinned to OpenCV float semantics
 and `colorsys` instead.
 

@@ -50,17 +50,23 @@ def test_no_cpu_fallback():
         rbunet.confusion_counts(torch.rand((1, 4)), torch.rand((1, 4)))
 
 
-def test_state_dict_schema_and_init_match_the_reference_schema():
+def test_state_dict_schema_and_init_match_the_reference_schema(golden_dir):
+    import numpy as np
     import torch
     import rbunet
     from oracle import robust_unet_ref as R
-    for nc in (3, 4):
+    for nc, golden in ((3, "model_c3_b64_64x64.npz"), (4, "model_c4_b64_64x96.npz")):
         m = rbunet.RobustUNet(nc, 1, 64)
         sd = m.state_dict()
         shapes = R.robust_unet_shapes(nc, 1, 64)
         assert list(sd.keys()) == list(shapes.keys()) and len(sd) == 290
         for k, v in sd.items():
             assert tuple(v.shape) == tuple(shapes[k]), k
+        # the reference's parameter and running-statistics names in its registration order (recorded from
+        # Main_Final.RobustUNet by oracle/make_golden.py): the same order draws the same initial weights under one seed
+        g = np.load(os.path.join(golden_dir, golden))
+        assert [n for n, _ in m.named_parameters()] == [str(n) for n in g["param_names"]]
+        assert [n for n in sd if n.endswith(("running_mean", "running_var"))] == [str(n) for n in g["buffer_names"]]
     assert sum(p.numel() for p in rbunet.RobustUNet(3).parameters()) == 40872223      # SURVEY.md §2
 
 

@@ -2,7 +2,7 @@
 shapes -- rbunet.RobustUNet through nn.Module -> C ABI -> sm_100a kernels against
 
   (a) goldens produced by the UNMODIFIED reference at base 64 (tests/golden/model_c*_b64_*.npz),
-  (b) the fp32 CPU oracle (bit-identical to Main_Final.RobustUNet, tests/test_oracle_vs_reference.py) on the same
+  (b) the fp32 CPU oracle (pinned to the reference's goldens, tests/test_oracle_golden.py) on the same
       weights, inputs and injected Dropout2d masks (Main_Final.py:226-321,573-582), and
   (c) the yardstick: torch's OWN `autocast(bfloat16)` execution of the reference arithmetic (eager ATen/cuDNN kernels on
       the same GPU, head + loss in fp32).
@@ -37,8 +37,8 @@ DEV = "cuda:0"
 
 
 def _reference_init_state_dict(nc):
-    """The reference's own initialisation (torch.manual_seed(0); RobustUNet(nc, 1) -- bit-identical to
-    Main_Final.RobustUNet under the same seed, tests/test_oracle_vs_reference.py) as a CPU state_dict."""
+    """The reference's own initialisation (torch.manual_seed(0); RobustUNet(nc, 1) -- the parameter registration order of
+    Main_Final.RobustUNet, hence its initial weights under the same seed) as a CPU state_dict."""
     import rbunet
     torch.manual_seed(0)
     m = rbunet.RobustUNet(nc, 1, 64)

@@ -8,6 +8,19 @@ import torch
 
 from oracle import robust_unet_ref as R
 
+GOLDEN_THREADS = 8       # torch.set_num_threads of oracle/make_golden.py
+
+
+@pytest.fixture(autouse=True)
+def golden_thread_count():
+    """torch's CPU convolutions split their sums by the intra-op thread count, so the oracle reproduces the goldens bit for
+    bit only with the thread count that wrote them, whatever the host's core count (elsewhere: up to 1.6e-4 on the eval
+    probabilities of model_c4_b16_32x48)."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
 
 def _load(golden_dir, name):
     return np.load(os.path.join(golden_dir, name), allow_pickle=False)

@@ -1,6 +1,6 @@
 """CPU: the numpy restatement of the reference's image operations (oracle/imageops_ref.py) against the committed
 fixtures generated from the reference's own enhance_image and from OpenCV (tests/golden/imageops.npz), against numpy's
-percentile, and -- when the build container's reference tree / cv2 are present -- against the live code."""
+percentile, and -- when cv2 is installed -- against live OpenCV."""
 import os
 
 import numpy as np
@@ -62,17 +62,3 @@ def test_against_live_opencv_when_present():
         m = ((rng.random((37, 53)) > 0.93) * 255).astype(np.uint8)
         ref = cv2.dilate(m, cv2.getStructuringElement(cv2.MORPH_ELLIPSE, (k, k)), iterations=1) - m
         assert np.array_equal(I.coastline_mask(m, k), ref)
-
-
-def test_against_live_reference_when_present():
-    from oracle import load_reference as L
-    if not L.reference_available():
-        pytest.skip("reference tree not present (GPU box)")
-    import importlib
-    L.load_reference()
-    T = importlib.import_module("tif_to_image")
-    conv = T.TIFToImageConverter.__new__(T.TIFToImageConverter)
-    rng = np.random.default_rng(3)
-    rgb = np.clip(rng.gamma(2.0, 2500.0, size=(40, 30, 3)), 0, 65535).astype(np.uint16)
-    for ew in (True, False):
-        assert np.array_equal(I.enhance_image(rgb, ew), conv.enhance_image(rgb, ew).astype(np.uint8))
