@@ -12,10 +12,10 @@ from . import _lib  # noqa: F401
 from .loss import (METRIC_KEYS, RobustBCEDiceLoss, batch_metrics, calculate_metrics,  # noqa: F401
                    confusion_counts, metrics_from_counts)
 from .model import AttentionGate, DilatedBlock, ResidualBlock, RobustUNet  # noqa: F401
-from .ops import View, coastline_mask, enhance_image, preprocess  # noqa: F401
+from .ops import View, coastline_mask, enhance_image, preprocess, resize  # noqa: F401
 from .optim import FusedAdam  # noqa: F401
 from .parallel import DataParallel, GradBucketer  # noqa: F401
 from .unet import CrossEntropyArgmaxLoss, UNet  # noqa: F401
 
 __all__ = ["RobustUNet", "ResidualBlock", "AttentionGate", "DilatedBlock", "RobustBCEDiceLoss", "calculate_metrics", "batch_metrics", "confusion_counts",
-           "metrics_from_counts", "METRIC_KEYS", "View", "preprocess", "enhance_image", "coastline_mask", "DataParallel", "GradBucketer", "FusedAdam", "UNet", "CrossEntropyArgmaxLoss"]
+           "metrics_from_counts", "METRIC_KEYS", "View", "preprocess", "resize", "enhance_image", "coastline_mask", "DataParallel", "GradBucketer", "FusedAdam", "UNet", "CrossEntropyArgmaxLoss"]

@@ -147,9 +147,17 @@ def confusion_counts(pred, target, threshold=0.5):
     return counts
 
 
-def preprocess(img_u8: torch.Tensor, n_channels: int = 3) -> torch.Tensor:
+def preprocess(img_u8, n_channels: int = 3, size=None) -> torch.Tensor:
     """uint8 RGB [B,H,W,3] CUDA tensor -> fp32 NCHW [B,n_channels,H,W] (Normalize of Main_Final.py:697-701; channels
-    beyond 3 are the build-defined HSV planes)."""
+    beyond 3 are the build-defined HSV planes).  With `size`, the images are first resized by `resize(img_u8, size)`
+    (Pillow bilinear = torchvision Resize on PIL images): the reference's Compose([Resize(size), ToTensor(), Normalize]).
+    `img_u8` may then also be an RGB [H,W,3] image or a list of RGB images of different sizes.  (Two launches: a fused
+    single-pass form measured slower on B200, profiles/r03_resize_fused_ab.txt.)"""
+    if size is not None:
+        srcs, _, C, _ = _resize_sources(img_u8, "rbunet.preprocess")
+        if C != 3:
+            raise RuntimeError("rbunet.preprocess expects RGB images [..., 3]")
+        img_u8 = resize(srcs, size)
     if not img_u8.is_cuda or img_u8.dtype != torch.uint8 or img_u8.dim() != 4 or img_u8.shape[-1] != 3:
         raise RuntimeError("rbunet.preprocess expects a uint8 CUDA tensor [B,H,W,3] (no CPU fallback)")
     img_u8 = img_u8.contiguous()
@@ -157,6 +165,97 @@ def preprocess(img_u8: torch.Tensor, n_channels: int = 3) -> torch.Tensor:
     out = torch.empty((B, n_channels, H, W), dtype=torch.float32, device=img_u8.device)
     call("rbu_preprocess", _p(img_u8), B, H, W, n_channels, _p(out), stream_ptr())
     return out
+
+
+_RESIZE_MODES = {"bilinear": 0, "nearest": 1, "cv2_nearest": 2}
+_DESC = None
+
+
+def _resize_sources(images, who):
+    """Normalise `images` to a list of [H,W,C] uint8 CUDA views (C 1 or 3, dense pixels, rows may be strided)."""
+    single = False
+    if isinstance(images, torch.Tensor):
+        if images.dim() == 2 or (images.dim() == 3 and images.shape[-1] == 3):
+            images, single = [images], True
+        elif images.dim() in (3, 4):
+            images = list(images.unbind(0))
+        else:
+            raise RuntimeError(f"{who} expects [H,W], [H,W,3], [B,H,W] or [B,H,W,3] uint8 CUDA tensors")
+    images = list(images)
+    if not images:
+        raise RuntimeError(f"{who}: no images")
+    srcs = []
+    for im in images:
+        if not isinstance(im, torch.Tensor) or not im.is_cuda or im.dtype != torch.uint8 or im.dim() not in (2, 3):
+            raise RuntimeError(f"{who} expects uint8 CUDA images [H,W] or [H,W,3] (no CPU fallback)")
+        x = im.unsqueeze(-1) if im.dim() == 2 else im
+        if x.shape[2] not in (1, 3) or x.shape[0] <= 0 or x.shape[1] <= 0:
+            raise RuntimeError(f"{who}: images must be non-empty with 1 or 3 bands, got {tuple(im.shape)}")
+        if not ((x.shape[2] == 1 or x.stride(2) == 1) and (x.shape[1] == 1 or x.stride(1) == x.shape[2])):
+            raise RuntimeError(f"{who}: the pixels of a row must be dense (rows may be strided)")
+        srcs.append(x)
+    if len({x.shape[2] for x in srcs}) != 1 or len({x.device for x in srcs}) != 1:
+        raise RuntimeError(f"{who}: all images must have the same band count and device")
+    return srcs, srcs[0].device, srcs[0].shape[2], single
+
+
+def _output_size(srcs, size, who):
+    """(oh, ow) shared by every source: (h, w) as given, or torchvision's Resize(int) rule (shorter side = size)."""
+    if isinstance(size, int):
+        sizes = set()
+        for x in srcs:
+            h, w = x.shape[0], x.shape[1]
+            short, long = (w, h) if w <= h else (h, w)
+            new_long = int(size * long / short)
+            sizes.add((new_long, size) if w <= h else (size, new_long))
+        if len(sizes) != 1:
+            raise RuntimeError(f"{who}: Resize({size}) gives images of different sizes {sorted(sizes)}; pass (h, w)")
+        oh, ow = sizes.pop()
+    else:
+        oh, ow = (int(v) for v in size)
+    if oh <= 0 or ow <= 0:
+        raise RuntimeError(f"{who}: output size must be positive, got {(oh, ow)}")
+    return oh, ow
+
+
+def _descriptor_table(srcs, dev):
+    """rbu_resize_src[B] on the device, copied from a pinned host buffer on the current stream (no synchronisation)."""
+    import numpy as np
+    global _DESC
+    if _DESC is None:
+        _DESC = np.dtype([("src", "<u8"), ("row_pitch", "<i8"), ("H", "<i4"), ("W", "<i4")])
+    tab = np.zeros(len(srcs), _DESC)
+    tab["src"] = [x.data_ptr() for x in srcs]
+    tab["row_pitch"] = [x.stride(0) for x in srcs]
+    tab["H"] = [x.shape[0] for x in srcs]
+    tab["W"] = [x.shape[1] for x in srcs]
+    host = torch.empty(tab.nbytes, dtype=torch.uint8, pin_memory=True)
+    host.numpy()[:] = tab.view(np.uint8)
+    with torch.cuda.device(dev):
+        table = host.to(dev, non_blocking=True)
+    return table, int(tab["H"].max()), int(tab["W"].max())
+
+
+def resize(images, size, interpolation: str = "bilinear") -> torch.Tensor:
+    """Resize uint8 CUDA images or masks, bit-exact with the reference's library calls:
+      "bilinear"     Pillow Image.resize(BILINEAR) = torchvision transforms.Resize on PIL images (Main_Final.py:697-701)
+      "nearest"      Pillow Image.resize(NEAREST), the mask resize of Main_Final.py:44-54
+      "cv2_nearest"  cv2.resize(INTER_NEAREST), the predicted mask back to scene size (predict_coastline.py:583-602)
+    `images`: [H,W], [H,W,3], [B,H,W] or [B,H,W,3], or a list of [H,W] / [H,W,3] images of different sizes (rows may be
+    strided, pixels dense).  `size`: (h, w), or an int for torchvision's shorter-side rule.  Returns uint8 [B,h,w(,3)]
+    from one launch, or one image when one image came in."""
+    if interpolation not in _RESIZE_MODES:
+        raise RuntimeError(f"rbunet.resize: interpolation must be one of {sorted(_RESIZE_MODES)}")
+    srcs, dev, C, single = _resize_sources(images, "rbunet.resize")
+    oh, ow = _output_size(srcs, size, "rbunet.resize")
+    table, max_h, max_w = _descriptor_table(srcs, dev)
+    out = torch.empty((len(srcs), oh, ow, C), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        call("rbu_resize_u8", _p(table), len(srcs), C, max_h, max_w, oh, ow, _RESIZE_MODES[interpolation], _p(out),
+             stream_ptr(), nbytes=float(sum(s.numel() for s in srcs) + out.numel()))
+    if C == 1:
+        out = out[..., 0]
+    return out[0] if single else out
 
 
 def enhance_image(img: torch.Tensor, enhance_water: bool = True, return_percentiles: bool = False):

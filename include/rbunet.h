@@ -63,6 +63,21 @@ int rbu_enhance_image(const void* img, int bits, int B, int H, int W, int C, int
  * iterations=1) - mask on uint8 [B,H,W] masks (any values; uint8 arithmetic), 1 <= ksize <= 64.  Contour tracing
  * (cv2.findContours / approxPolyDP, :605-616) stays on the host. */
 int rbu_coastline_mask(const uint8_t* mask, int B, int H, int W, int ksize, uint8_t* out, void* stream);
+/* Resizing of uint8 images (C = 3, RGB) and masks (C = 1), bit-exact with the library calls of the reference.  One
+ * launch per call for a batch of sources of different sizes, all resized to oh x ow.  srcs_device: DEVICE array of B
+ * descriptors (row_pitch in bytes >= W*C; the C bytes of a pixel are contiguous).  max_h / max_w bound every source's
+ * H / W and size the bilinear weight tables; a descriptor outside them is skipped (its output is left unwritten).
+ * out: [B,oh,ow,C] uint8.
+ *  mode 0  Pillow Image.resize(BILINEAR) = torchvision transforms.Resize on PIL images (Main_Final.py:697-701,
+ *          predict_coastline.py:386-392): Pillow's antialiasing two-pass fixed-point filter.  Downscales needing more
+ *          than RBU_RESIZE_MAX_TAPS taps per output (factor > 127) return RBU_ERR_UNSUPPORTED.
+ *  mode 1  Pillow Image.resize(NEAREST): the mask resize of Main_Final.py:44-54.
+ *  mode 2  cv2.resize(INTER_NEAREST): the predicted mask back to scene size (predict_coastline.py:583-602).
+ * Pinned against Pillow 12.2, OpenCV 4.13 and torchvision 0.26. */
+#define RBU_RESIZE_MAX_TAPS (255)
+typedef struct { const uint8_t* src; long long row_pitch; int H, W; } rbu_resize_src;
+int rbu_resize_u8(const rbu_resize_src* srcs_device, int B, int C, int max_h, int max_w, int oh, int ow, int mode,
+                  uint8_t* out, void* stream);
 
 /* ------------------------------------------------------------------ tensor-core implicit GEMM
  * Replaces aten::convolution for 3x3 (dilation 1/2/4), 1x1 and ConvTranspose2d(2, stride 2)
