@@ -1099,6 +1099,19 @@ int colsum_fold(const float*& part, int& nblk, long& stride, int K, float* scrat
 #define CH_OK(C) ((C) >= 8 && (C) <= 2048 && pow2(C))
 #define FOLD_FLOATS(K) ((size_t)COLSUM_SLICES * (K))
 
+size_t colsum_scratch_floats(int K) { return FOLD_FLOATS(K); }
+
+int colsum_split(const float* part, int nblk, long stride, int K1, float* out1, int K2, float* out2, float* scratch,
+                 cudaStream_t st) {
+  int rc = colsum_fold(part, nblk, stride, K1 + K2, scratch, st);
+  if (rc) return rc;
+  colsum_kernel<<<rbu_cdiv(K1, 32), 256, 0, st>>>(part, nblk, K1, stride, out1, 1.f);
+  RBU_CHECK_LAUNCH();
+  colsum_kernel<<<rbu_cdiv(K2, 32), 256, 0, st>>>(part + K1, nblk, K2, stride, out2, 1.f);
+  RBU_CHECK_LAUNCH();
+  return RBU_OK;
+}
+
 // Workspace (floats) large enough for every backward pass of a [N,HW,C] tensor: max partial layout is
 // [N*chunks][4][C] (AttentionGate pass 2); the head / chan_sum layouts are smaller.
 extern "C" size_t rbu_bwd_workspace_bytes(int N, int HW, int C) {

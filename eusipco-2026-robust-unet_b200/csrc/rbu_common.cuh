@@ -56,6 +56,13 @@ static inline int rbu_cdiv(long a, long b) { return (int)((a + b - 1) / b); }
 // resident warps per SM over a few waves are useful.  `per_iter` = items one block covers per loop iteration (threads x U).
 int rbu_stream_blocks(long items_per_image, int per_iter, int images);
 
+// Deterministic column sums of per-CTA partial rows part[nblk][stride] (backward_ops.cu): out1[k] = sum of column k for
+// k < K1, out2[k] = sum of column K1 + k for k < K2 (fixed order, double accumulation).  Long lists are first folded in
+// `scratch`, which must hold colsum_scratch_floats(K1 + K2) floats.
+size_t colsum_scratch_floats(int K);
+int colsum_split(const float* part, int nblk, long stride, int K1, float* out1, int K2, float* out2, float* scratch,
+                 cudaStream_t st);
+
 // ---------------------------------------------------------------------------------------------
 // device helpers
 // ---------------------------------------------------------------------------------------------

@@ -782,10 +782,16 @@ class Engine:
             keep(f"dec{k}", st)
             del st, cat, skip
         P = N * H * W
-        probs = torch.empty((N, 1, H, W), dtype=torch.float32, device=dev)
         hc = m.outc[0]
+        K = hc.out_channels
+        probs = torch.empty((N, K, H, W), dtype=torch.float32, device=dev)
         logits = torch.empty_like(probs) if self.keep_logits else None
-        call("rbu_head_forward", _vp(cur), cur.ld, P, cur.C, _p(hc.weight), _p(hc.bias), _p(probs), _p(logits), stream_ptr())
+        if K == 1:
+            call("rbu_head_forward", _vp(cur), cur.ld, P, cur.C, _p(hc.weight), _p(hc.bias), _p(probs), _p(logits),
+                 stream_ptr())
+        else:                                      # a sigmoid per class, as the reference's outc
+            call("rbu_headk_forward", _vp(cur), cur.ld, P, H * W, cur.C, K, _p(hc.weight), _p(hc.bias), 1, _p(probs),
+                 _p(logits), stream_ptr())
         self.last_logits = logits
         S["head_x"] = cur
         S["probs"] = probs
@@ -807,9 +813,15 @@ class Engine:
         hc = m.outc[0]
         d = self.new(N, H, W, hx.C, dev)
         gw, gb = torch.empty_like(hc.weight), torch.empty_like(hc.bias)
-        ws = self.bwd_ws(N, H * W, hx.C, dev)
-        call("rbu_head_backward", _p(dprobs.contiguous()), _p(S["probs"]), _vp(hx), hx.ld, _vp(d), d.ld, P, hx.C,
-             _p(hc.weight), _p(gw), _p(gb), _p(ws), ws.numel() * 4, stream_ptr())
+        K = hc.out_channels
+        if K == 1:
+            ws = self.bwd_ws(N, H * W, hx.C, dev)
+            call("rbu_head_backward", _p(dprobs.contiguous()), _p(S["probs"]), _vp(hx), hx.ld, _vp(d), d.ld, P, hx.C,
+                 _p(hc.weight), _p(gw), _p(gb), _p(ws), ws.numel() * 4, stream_ptr())
+        else:
+            ws = self.ws(_lib.lib().rbu_headk_backward_workspace_bytes(P, hx.C, K), dev)
+            call("rbu_headk_backward", _p(dprobs.contiguous()), _p(S["probs"]), _vp(hx), hx.ld, _vp(d), d.ld, P, H * W,
+                 hx.C, K, 1, _p(hc.weight), _p(gw), _p(gb), _p(ws), ws.numel() * 4, stream_ptr())
         grads["outc.0.weight"], grads["outc.0.bias"] = gw, gb
 
         def done(*prefixes):

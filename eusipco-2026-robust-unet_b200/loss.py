@@ -78,3 +78,24 @@ def batch_metrics(pred: torch.Tensor, target: torch.Tensor, threshold: float = 0
     """Per-image metric dicts for a whole batch with ONE device->host copy of [B,4] counts (the reference
     copies every image to the host, Main_Final.py:604-606,655-657)."""
     return [metrics_from_counts(*c) for c in confusion_counts(pred, target, threshold).cpu().tolist()]
+
+
+def class_confusion_counts(pred: torch.Tensor, target: torch.Tensor, threshold: float = 0.5) -> torch.Tensor:
+    """[B,K,H,W] per-class probabilities (a K-class RobustUNet's output) / 0-1 masks on the GPU -> int64 [B,K,4] =
+    TP, FP, FN, TN of each class (pred > threshold, strict), from one counting pass over the B*K planes."""
+    if not pred.is_cuda:
+        raise RuntimeError("rbunet.class_confusion_counts runs on CUDA tensors only (no CPU fallback)")
+    if pred.dim() < 3 or pred.shape != target.shape:
+        raise ValueError(f"expected pred and target of the same shape [B,K,H,W], got {tuple(pred.shape)} and "
+                         f"{tuple(target.shape)}")
+    B, K = pred.shape[0], pred.shape[1]
+    if B * K > 65535:
+        raise ValueError(f"B*K = {B * K} planes; at most 65535 per call")
+    p = pred.detach().contiguous().float().reshape(B * K, -1)
+    t = target.detach().contiguous().float().reshape(B * K, -1)
+    return ops.confusion_counts(p, t, threshold).reshape(B, K, 4)
+
+
+def class_metrics(pred: torch.Tensor, target: torch.Tensor, threshold: float = 0.5) -> list:
+    """For each image, K metric dicts (metrics_from_counts of each class plane) with ONE device->host copy."""
+    return [[metrics_from_counts(*c) for c in img] for img in class_confusion_counts(pred, target, threshold).cpu().tolist()]

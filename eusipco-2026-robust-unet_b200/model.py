@@ -2,7 +2,8 @@
 
 `RobustUNet(n_channels=3, n_classes=1, base_channels=64)` has the constructor, parameter registration
 order (hence identical initial weights under the same `torch.manual_seed`), the 290 `state_dict` keys /
-shapes / dtypes and the `forward(x) -> probabilities [B,1,H,W]` contract of the reference model
+shapes / dtypes and the `forward(x) -> probabilities [B,K,H,W]` contract (K = n_classes, 1 <= K <= 32: a sigmoid per
+class, as the reference's `outc`) of the reference model
 (Main_Final.py:226-321), so reference checkpoints load unchanged and an unmodified
 `torch.optim.Adam(model.parameters())` + `loss.backward()` loop (Main_Final.py:552,573-582) trains it.
 
@@ -222,11 +223,13 @@ class RobustUNet(nn.Module):
 
     def __init__(self, n_channels=3, n_classes=1, base_channels=64):
         super().__init__()
-        if n_classes != 1:
-            raise ValueError("the fused sigmoid head supports n_classes == 1 (every reference call site uses 1)")
+        if not 1 <= n_classes <= 32:
+            raise ValueError(f"n_classes must be in [1, 32], got {n_classes}")
         b = base_channels
         if b < 16 or b & (b - 1):
             raise ValueError("base_channels must be a power of two >= 16")
+        if n_classes > 1 and b > 256:
+            raise ValueError("the K-class head takes at most 256 input channels: base_channels <= 256 when n_classes > 1")
         self.inc = ResidualBlock(n_channels, b, 0.1)
         self.down1 = nn.Sequential(_Slot(), ResidualBlock(b, 2 * b, 0.1))
         self.down2 = nn.Sequential(_Slot(), ResidualBlock(2 * b, 4 * b, 0.2))

@@ -3,9 +3,10 @@
 argmax accuracy / IoU (:384-388), on the same sm_100a kernels as the Robust U-Net.
 
 `rbunet.UNet(n_channels=3, n_classes=2)` has the reference's constructor, parameter registration order, the 136
-`state_dict` keys and `forward(x) -> logits [B,2,H,W]`; `rbunet.CrossEntropyArgmaxLoss()` is interchangeable with
-`nn.CrossEntropyLoss()` on those logits and also leaves the per-image argmax confusion counts in `last_counts`
-(torch's own `nn.CrossEntropyLoss` works on the logits too).  No CPU fallback.
+`state_dict` keys and `forward(x) -> logits [B,K,H,W]` (K = n_classes, 1 <= K <= 32); `rbunet.CrossEntropyArgmaxLoss()`
+is interchangeable with `nn.CrossEntropyLoss()` on those logits (2 <= K <= 32) and also leaves the per-image argmax
+confusion counts in `last_counts` (class 1 against the rest) and `last_class_counts` (every class).  Torch's own losses
+work on the logits too (`nn.BCEWithLogitsLoss` at K = 1).  No CPU fallback.
 """
 from __future__ import annotations
 
@@ -187,9 +188,14 @@ class UNetEngine(Engine):
             else:
                 cats[lvl] = None
             del st, cat
-        logits = torch.empty((N, 2, H, W), dtype=torch.float32, device=dev)
-        call("rbu_head2_forward", _vp(cur), cur.ld, N * H * W, H * W, cur.C, _p(m.final.weight), _p(m.final.bias), _p(logits),
-             stream_ptr())
+        K = m.final.out_channels
+        logits = torch.empty((N, K, H, W), dtype=torch.float32, device=dev)
+        if K == 2:
+            call("rbu_head2_forward", _vp(cur), cur.ld, N * H * W, H * W, cur.C, _p(m.final.weight), _p(m.final.bias),
+                 _p(logits), stream_ptr())
+        else:
+            call("rbu_headk_forward", _vp(cur), cur.ld, N * H * W, H * W, cur.C, K, _p(m.final.weight), _p(m.final.bias), 0,
+                 _p(logits), NULL, stream_ptr())
         if save:
             S["cats"] = cats
             S["head_x"] = cur
@@ -203,10 +209,16 @@ class UNetEngine(Engine):
         hx = S["head_x"]
         d = self.new(N, H, W, hx.C, dev)
         gw, gb = torch.empty_like(m.final.weight), torch.empty_like(m.final.bias)
-        nbytes = _lib.lib().rbu_head2_backward_workspace_bytes(N * H * W, hx.C)
-        ws = self.ws(nbytes, dev)
-        call("rbu_head2_backward", _p(dlogits.contiguous()), _vp(hx), hx.ld, _vp(d), d.ld, N * H * W, H * W, hx.C,
-             _p(m.final.weight), _p(gw), _p(gb), _p(ws), ws.numel() * 4, stream_ptr())
+        K = m.final.out_channels
+        if K == 2:
+            nbytes = _lib.lib().rbu_head2_backward_workspace_bytes(N * H * W, hx.C)
+            ws = self.ws(nbytes, dev)
+            call("rbu_head2_backward", _p(dlogits.contiguous()), _vp(hx), hx.ld, _vp(d), d.ld, N * H * W, H * W, hx.C,
+                 _p(m.final.weight), _p(gw), _p(gb), _p(ws), ws.numel() * 4, stream_ptr())
+        else:
+            ws = self.ws(_lib.lib().rbu_headk_backward_workspace_bytes(N * H * W, hx.C, K), dev)
+            call("rbu_headk_backward", _p(dlogits.contiguous()), NULL, _vp(hx), hx.ld, _vp(d), d.ld, N * H * W, H * W,
+                 hx.C, K, 0, _p(m.final.weight), _p(gw), _p(gb), _p(ws), ws.numel() * 4, stream_ptr())
         grads["final.weight"], grads["final.bias"] = gw, gb
         denc = {}
         for lvl, C in self.LEVELS:
@@ -268,8 +280,8 @@ class UNet(nn.Module):
 
     def __init__(self, n_channels=3, n_classes=2):
         super().__init__()
-        if n_classes != 2:
-            raise ValueError("the fused two-logit head supports n_classes == 2 (every reference call site uses 2)")
+        if not 1 <= n_classes <= 32:
+            raise ValueError(f"n_classes must be in [1, 32], got {n_classes}")
         self.enc1 = _conv_block(n_channels, 64)
         self.enc2 = _conv_block(64, 128)
         self.enc3 = _conv_block(128, 256)
@@ -318,24 +330,86 @@ class _CE2(torch.autograd.Function):
         return dz, None, None
 
 
+class _CEK(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, logits, target, mod):
+        z = logits.detach().contiguous().float()
+        t = target.detach().contiguous().long()
+        B, K, HW = z.shape[0], z.shape[1], z.shape[2] * z.shape[3]
+        dev = z.device
+        nbytes = _lib.lib().rbu_cek_workspace_bytes(B, HW, K)
+        ws = torch.empty((nbytes + 7) // 8, dtype=torch.int64, device=dev)
+        loss = torch.empty(1, dtype=torch.float32, device=dev)
+        counts = torch.empty((B, K, 4), dtype=torch.int64, device=dev)
+        invalid = torch.empty(1, dtype=torch.int64, device=dev)
+        call("rbu_cek_forward", _p(z), _p(t), B, HW, K, _p(ws), ws.numel() * 8, _p(loss), _p(counts), _p(invalid),
+             stream_ptr())
+        mod.last_counts = counts[:, 1]
+        mod._class_counts = counts
+        mod._invalid = invalid
+        ctx.save_for_backward(z, t)
+        return loss.reshape(())
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        z, t = ctx.saved_tensors
+        B, K, HW = z.shape[0], z.shape[1], z.shape[2] * z.shape[3]
+        dz = torch.empty_like(z)
+        g = grad_out.detach().contiguous().float().reshape(1)
+        call("rbu_cek_backward", _p(z), _p(t), B, HW, K, _p(g), _p(dz), stream_ptr())
+        return dz, None, None
+
+
 class CrossEntropyArgmaxLoss(nn.Module):
-    """= nn.CrossEntropyLoss() on [B,2,H,W] logits and [B,H,W] class indices (train_water_segmentation.py:304,381);
-    `last_counts` holds the per-image TP/FP/FN/TN of argmax == 1 vs target == 1 (:384-388)."""
+    """= nn.CrossEntropyLoss() on [B,K,H,W] logits (2 <= K <= 32) and [B,H,W] class indices
+    (train_water_segmentation.py:304,381).  `last_counts` holds the per-image TP/FP/FN/TN of argmax == 1 vs target == 1
+    (:384-388), `last_class_counts` the same [B,K,4] for every class (arg-max ties go to the lowest class index).
+
+    At K = 2 any nonzero target is class 1, as in the two-class kernel.  For K > 2 a target outside [0, K) adds no loss
+    and no counts (the loss is still divided by B*H*W); the methods that read counts to the host then raise ValueError.
+    `forward` never synchronises."""
 
     def __init__(self):
         super().__init__()
         self.last_counts = None
+        self._class_counts = None
+        self._invalid = None
 
     def forward(self, logits, target):
         if not logits.is_cuda or not target.is_cuda:
             raise RuntimeError("rbunet.CrossEntropyArgmaxLoss runs on CUDA tensors only (no CPU fallback)")
-        if logits.dim() != 4 or logits.shape[1] != 2 or tuple(target.shape) != (logits.shape[0],) + tuple(logits.shape[2:]):
-            raise ValueError("expected logits [B,2,H,W] and class-index targets [B,H,W]")
-        return _CE2.apply(logits, target, self)
+        if logits.dim() != 4 or not 2 <= logits.shape[1] <= 32 or \
+                tuple(target.shape) != (logits.shape[0],) + tuple(logits.shape[2:]):
+            raise ValueError(f"expected logits [B,K,H,W] with 2 <= K <= 32 and class-index targets [B,H,W], got "
+                             f"{tuple(logits.shape)} and {tuple(target.shape)}")
+        if logits.shape[1] == 2:
+            self._class_counts = self._invalid = None
+            return _CE2.apply(logits, target, self)
+        return _CEK.apply(logits, target, self)
+
+    @property
+    def last_class_counts(self):
+        """int64 [B,K,4] TP/FP/FN/TN of each class (device tensor); at K = 2 class 0 is [TN, FN, FP, TP] of class 1."""
+        if self._class_counts is None and self.last_counts is not None:
+            c = self.last_counts
+            return torch.stack([c.flip(1), c], dim=1)
+        return self._class_counts
+
+    def _host_counts(self):
+        if self._invalid is not None:
+            n = int(self._invalid.item())
+            if n:
+                raise ValueError(f"{n} target pixels are outside [0, {self._class_counts.shape[1]}): no counts for them")
+        return self.last_class_counts.sum(0).cpu().tolist()
 
     def batch_accuracy_iou(self):
-        """accuracy and IoU over the whole batch as WaterSegmentationTrainer.validate_model computes them
-        (:384-388, calculate_iou :341-358: union == 0 -> 1.0)."""
-        tp, fp, fn, tn = [float(v) for v in self.last_counts.sum(0).cpu().tolist()]
+        """accuracy and IoU of class 1 over the whole batch as WaterSegmentationTrainer.validate_model computes them
+        (:384-388, calculate_iou :341-358: union == 0 -> 1.0); accuracy is the pixel accuracy of the K-class arg-max."""
+        cc = self._host_counts()
+        tp, fp, fn, _ = [float(v) for v in cc[1]]
         union = tp + fp + fn
-        return (tp + tn) / (tp + fp + fn + tn), (1.0 if union == 0 else tp / union)
+        return float(sum(c[0] for c in cc)) / float(sum(cc[0])), (1.0 if union == 0 else tp / union)
+
+    def class_iou(self):
+        """K IoUs over the whole batch, union == 0 -> 1.0 (calculate_iou, :341-358)."""
+        return [1.0 if tp + fp + fn == 0 else float(tp) / float(tp + fp + fn) for tp, fp, fn, _ in self._host_counts()]

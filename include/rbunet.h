@@ -327,6 +327,31 @@ int rbu_ce2_forward(const float* logits, const int64_t* target, int B, int64_t H
 int rbu_ce2_backward(const float* logits, const int64_t* target, int B, int64_t HW, const float* grad_out, float* dlogits,
                      void* stream);
 
+/* ------------------------------------------------------------------ K-class heads (1 <= K <= 32)
+ * RobustUNet's outc = Conv2d(b, n_classes, 1) + Sigmoid (Main_Final.py:274-277) and UNet's final = Conv2d(64, n_classes, 1)
+ * trained with nn.CrossEntropyLoss (train_water_segmentation.py:246,288,304) for any class count.  RobustUNet with K = 1
+ * keeps rbu_head_*, UNet with K = 2 keeps rbu_head2_* / rbu_ce2_*.  C is a power of two in [16, 256]; P % HW == 0.
+ *
+ * K-output 1x1 head: out[n][k][hw] = w[k].x[p] + b[k], fp32 NCHW [N][K][HW]; sigmoid != 0 applies the same
+ * sigmoidf_acc as rbu_head_forward (RobustUNet outc); logits (optional) receives the pre-sigmoid values. */
+int rbu_headk_forward(const void* x, int64_t ld, int64_t P, int HW, int C, int K, const float* w, const float* b,
+                      int sigmoid, float* out, float* logits, void* stream);
+size_t rbu_headk_backward_workspace_bytes(int64_t P, int C, int K);
+/* dz = sigmoid ? dout*p*(1-p) (as rbu_head_backward) : dout;  dx = sum_k dz_k w_k (bf16 view);
+ * dw[K][C] = sum_p dz x;  db[K] = sum_p dz  -- two-stage, fixed order, no float atomics */
+int rbu_headk_backward(const float* dout, const float* probs, const void* x, int64_t x_ld, void* dx, int64_t dx_ld,
+                       int64_t P, int HW, int C, int K, int sigmoid, const float* w, float* dw, float* db,
+                       void* workspace, size_t workspace_bytes, void* stream);
+/* nn.CrossEntropyLoss() over K classes + per-class argmax confusion counts [B][K][4] (TP, FP, FN, TN; ties -> lowest
+ * class index, as torch.argmax); targets outside [0, K) add no loss and no counts, and are counted in *invalid.  The
+ * loss is divided by B*HW.  B <= 65535. */
+size_t rbu_cek_workspace_bytes(int B, int64_t HW, int K);
+int rbu_cek_forward(const float* logits, const int64_t* target, int B, int64_t HW, int K, void* workspace,
+                    size_t workspace_bytes, float* loss_out, int64_t* class_counts, int64_t* invalid, void* stream);
+/* (softmax - onehot) * g / (B*HW); invalid pixels get 0 */
+int rbu_cek_backward(const float* logits, const int64_t* target, int B, int64_t HW, int K, const float* grad_out,
+                     float* dlogits, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
