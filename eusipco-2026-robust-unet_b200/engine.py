@@ -9,6 +9,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+from collections import namedtuple
 from ctypes import c_void_p
 
 import torch
@@ -16,10 +17,13 @@ import torch.nn as nn
 
 from . import _lib
 from ._lib import WgradArgs, call, stream_ptr
-from .ops import View, conv_gemm, pack_weight
+from .ops import View, conv_gemm, pack_dims, pack_weight
 
 BN_EPS = 1e-5
 NULL = c_void_p(0)
+
+# One row of rbu_pack_weights_multi's job table: _packs[key] <- src (and src2), see ops.pack_dims
+PackJob = namedtuple("PackJob", "key src src2 shape Nn T K mode cout")
 
 
 def _p(t):
@@ -105,8 +109,8 @@ class Engine:
         return self._ws.get(int(nbytes))
 
     def pack(self, param: torch.Tensor, mode: int):
-        """bf16 GEMM operand of a parameter.  Inside the whole-model path every operand has just been rebuilt by
-        refresh_packs(); standalone block calls (tests) pack on first use."""
+        """bf16 GEMM operand of a parameter (modes 0-3).  Inside the whole-model path every operand has just been rebuilt
+        by refresh_packs(); standalone block calls (tests) pack on first use."""
         key = (id(param), mode)
         ent = self._packs.get(key)
         if ent is None or ent.device != param.device:
@@ -114,76 +118,30 @@ class Engine:
             self._packs[key] = ent
         return ent
 
-    def pack_stem(self, w1, wsc, Kp):
-        key = (id(w1), "stem")
-        ent = self._packs.get(key)
-        if ent is None or ent.device != w1.device:
-            C, nc = w1.shape[0], w1.shape[1]
-            m = torch.zeros((2 * C, Kp), dtype=torch.float32, device=w1.device)
-            m[:C, :9 * nc] = w1.detach().permute(0, 2, 3, 1).reshape(C, 9 * nc)
-            m[C:, 4 * nc:5 * nc] = wsc.detach().reshape(C, nc)
-            ent = m.to(torch.bfloat16).reshape(2 * C, 1, Kp).contiguous()
-            self._packs[key] = ent
-        return ent
-
-    def _pack_plan(self):
-        """[(key, src, src2, dst shape, Nn, T, K, mode, Cout)] for every tensor-core weight operand of the model."""
+    def _packed_weights(self):
+        """[(weight, pack modes[, second source])]: every weight the network runs as a tensor-core GEMM operand, the stem
+        convolution first.  One of the three things a network supplies (with _network_forward / _network_backward)."""
         m = self.model
-        jobs = []
-
-        def conv(w, mode):
-            if mode == 0:
-                Nn, K, T = w.shape[0], w.shape[1], w.shape[2] * w.shape[3]
-            else:
-                Nn, K, T = w.shape[1], w.shape[0], w.shape[2] * w.shape[3]
-            jobs.append(((id(w), mode), w, None, (Nn, T, K), Nn, T, K, mode, 0))
-
-        nc = m.inc.conv1.in_channels
-        C0 = m.inc.conv1.out_channels
-        Kp = ((9 * nc + 7) // 8) * 8
-        jobs.append(((id(m.inc.conv1.weight), "stem"), m.inc.conv1.weight, m.inc.shortcut[0].weight, (2 * C0, 1, Kp),
-                     2 * C0, nc, Kp, 4, 0))
-        blocks = [m.inc, m.down1[1], m.down2[1], m.down3[1], m.bottleneck[2], m.dec4, m.dec3, m.dec2, m.dec1]
-        for blk in blocks:
-            stem = blk is m.inc
-            if not stem:
-                conv(blk.conv1.weight, 0)
-                conv(blk.conv1.weight, 1)
-            conv(blk.conv2.weight, 0)
-            conv(blk.conv2.weight, 1)
-            if not stem and not isinstance(blk.shortcut, nn.Identity):
-                conv(blk.shortcut[0].weight, 0)
-                conv(blk.shortcut[0].weight, 1)
-        for cv in (m.bottleneck[1].conv1, m.bottleneck[1].conv2, m.bottleneck[1].conv3, m.bottleneck[1].conv4):
-            conv(cv.weight, 0)
-            conv(cv.weight, 1)
-        for k in (4, 3, 2, 1):
-            gate = getattr(m, f"att{k}")
-            for cv in (gate.W_g[0], gate.W_x[0]):
-                conv(cv.weight, 0)
-                conv(cv.weight, 1)
-            w = getattr(m, f"up{k}").weight          # ConvTranspose2d [Cin, Cout, 2, 2]
-            jobs.append(((id(w), 2), w, None, (4 * w.shape[1], 1, w.shape[0]), 4 * w.shape[1], 1, w.shape[0], 2, w.shape[1]))
-            jobs.append(((id(w), 3), w, None, (w.shape[0], 4, w.shape[1]), w.shape[0], 4, w.shape[1], 3, 0))
-        return jobs
-
-    def _pack_src_params(self):
-        """The Parameter objects behind the packed operands, in a fixed order (identity check for the plan cache); None when
-        the model is not a RobustUNet."""
-        m = self.model
-        if not (hasattr(m, "inc") and hasattr(m, "att4")):
-            return None
-        out = [m.inc.conv1.weight, m.inc.shortcut[0].weight]
-        for blk in (m.inc, m.down1[1], m.down2[1], m.down3[1], m.bottleneck[2], m.dec4, m.dec3, m.dec2, m.dec1):
-            out += [blk.conv1.weight, blk.conv2.weight]
+        out = [(m.inc.conv1.weight, (4,), m.inc.shortcut[0].weight), (m.inc.conv2.weight, (0, 1))]
+        for blk in (m.down1[1], m.down2[1], m.down3[1], m.bottleneck[2], m.dec4, m.dec3, m.dec2, m.dec1):
+            out += [(blk.conv1.weight, (0, 1)), (blk.conv2.weight, (0, 1))]
             if not isinstance(blk.shortcut, nn.Identity):
-                out.append(blk.shortcut[0].weight)
+                out.append((blk.shortcut[0].weight, (0, 1)))
         d = m.bottleneck[1]
-        out += [d.conv1.weight, d.conv2.weight, d.conv3.weight, d.conv4.weight]
+        out += [(cv.weight, (0, 1)) for cv in (d.conv1, d.conv2, d.conv3, d.conv4)]
         for k in (4, 3, 2, 1):
             g = getattr(m, f"att{k}")
-            out += [g.W_g[0].weight, g.W_x[0].weight, getattr(m, f"up{k}").weight]
+            out += [(g.W_g[0].weight, (0, 1)), (g.W_x[0].weight, (0, 1)), (getattr(m, f"up{k}").weight, (2, 3))]
         return out
+
+    def _pack_plan(self):
+        """[PackJob] for every operand of _packed_weights(), in that order."""
+        jobs = []
+        for w, modes, *src2 in self._packed_weights():
+            for mode in modes:
+                Nn, T, K, cout, shape = pack_dims(w, mode)
+                jobs.append(PackJob((id(w), mode), w, src2[0] if src2 else None, shape, Nn, T, K, mode, cout))
+        return jobs
 
     def refresh_packs(self):
         """Rebuild every bf16 weight operand from the fp32 masters with ONE kernel launch.  Done at the start of every
@@ -193,18 +151,15 @@ class Engine:
         # the job list only depends on which Parameter objects the modules hold: rebuilt when one of them is replaced
         # (model.to(), load_state_dict(assign=True)), otherwise reused -- this runs on the launching thread before the
         # first kernel of every forward, i.e. while the GPU idles whenever the caller synchronised on the previous step
-        cur = self._pack_src_params()
-        if cur is None:                          # an engine without a cheap identity list (UNetEngine): rebuild every time
-            plan = self._pack_plan()
-        else:
-            srcs = self._pack_srcs
-            if srcs is None or len(srcs) != len(cur) or any(a is not b for a, b in zip(srcs, cur)):
-                self._pack_plan_cache = self._pack_plan()
-                self._pack_srcs = tuple(cur)
-            plan = self._pack_plan_cache
-        sig = tuple(j[1].data_ptr() for j in plan)
+        cur = tuple(t for w, _, *src2 in self._packed_weights() for t in (w, *src2))
+        srcs = self._pack_srcs
+        if srcs is None or len(srcs) != len(cur) or any(a is not b for a, b in zip(srcs, cur)):
+            self._pack_plan_cache = self._pack_plan()
+            self._pack_srcs = cur
+        plan = self._pack_plan_cache
+        sig = tuple(t.data_ptr() for t in cur)
         if self._pack_table is None or self._pack_table[0] != sig:
-            dev = plan[0][1].device
+            dev = plan[0].src.device
             dt = np.dtype([("src", "<u8"), ("src2", "<u8"), ("dst", "<u8"), ("first_block", "<i8"), ("total", "<i8"),
                            ("Nn", "<i4"), ("T", "<i4"), ("K", "<i4"), ("mode", "<i4"), ("Cout", "<i4"), ("reserved", "<i4")])
             tab = np.zeros(len(plan), dtype=dt)
@@ -413,9 +368,8 @@ class Engine:
         fuse = training and self.fuse_bn_stats
         if stem_patches is not None:
             y12 = self.new(N, H, W, 2 * C, dev)
-            wst = self.pack_stem(blk.conv1.weight, blk.shortcut[0].weight, stem_patches.C)
             st12 = self.conv_stats_buf(2 * C, dev) if fuse else None
-            conv_gemm(N, H, W, [(stem_patches, wst, 1, 0, False)], 2 * C, y12,
+            conv_gemm(N, H, W, [(stem_patches, self._packs[(id(blk.conv1.weight), 4)], 1, 0, False)], 2 * C, y12,
                       flops=2.0 * N * H * W * C * 10 * blk.conv1.in_channels, stats=st12)
             y1, ys = y12.slice(0, C), y12.slice(C, C)
             if fuse:
@@ -700,36 +654,75 @@ class Engine:
             grads[f"{prefix}.conv{i + 1}.bias"] = torch.zeros(Cq, device=dev)   # a bias before a train-mode BN
         return dx
 
-    # ------------------------------------------------------------------ whole model
+    # ------------------------------------------------------------------ ConvTranspose2d(2, stride 2) up-sampling
+    def up_forward(self, up, x: View, N, H, W, out: View):
+        """up(x) for x [N,H,W,Cin], scattered into out [N,2H,2W,Cout] (a channel slice of the decoder's concat buffer).
+        Returns the state up_backward needs."""
+        C = up.out_channels
+        conv_gemm(N, H, W, [(x, self.pack(up.weight, 2), 1, 0, False)], 4 * C, out, scatter=True, Cout=C, bias=up.bias)
+        return {"x": x, "N": N, "H": H, "W": W}
+
+    def up_backward(self, up, s, dout: View, grads: dict, prefix: str):
+        """Puts up's bias and weight gradients into grads; returns d(x)."""
+        N, H, W, x = s["N"], s["H"], s["W"], s["x"]
+        C, dev = dout.C, dout.base.device
+        gb = torch.empty_like(up.bias)
+        ws = self.bwd_ws(N, 4 * H * W, C, dev)
+        call("rbu_chan_sum", _vp(dout), dout.ld, 4 * N * H * W, C, _p(gb), _p(ws), ws.numel() * 4, stream_ptr())
+        dx = self.new(N, H, W, x.C, dev)
+        conv_gemm(N, H, W, [(dout, self.pack(up.weight, 3), 4, 0, True)], x.C, dx)
+        gw = self.gbuf(prefix + ".weight", up.weight)
+        self.wgrad(N, H, W, x, dout, 4, 0, True, gw)             # after the data gradient (see rb_backward)
+        grads[prefix + ".bias"], grads[prefix + ".weight"] = gb, gw
+        return dx
+
+    # ------------------------------------------------------------------ whole network
     def forward(self, x: torch.Tensor, training: bool, save: bool):
+        """The whole network on an NCHW input: (output [N,K,H,W] fp32, the state backward() needs if `save`, else None).
+        What differs between networks is _packed_weights and _network_forward."""
+        name = f"rbunet.{type(self.model).__name__}"
         if not x.is_cuda:
-            raise RuntimeError("rbunet.RobustUNet runs on CUDA tensors only (no CPU fallback)")
+            raise RuntimeError(f"{name} runs on CUDA tensors only (no CPU fallback)")
+        N, nc, H, W = x.shape
+        if H % 16 or W % 16:
+            raise RuntimeError(f"{name}: input H,W must be multiples of 16, got {H}x{W}")
         self._pending_counters = []
         self._defer_counters = True
         try:
             with torch.cuda.device(x.device):        # stream_ptr() and the library's per-device state follow the tensors
-                return self._forward_impl(x, training, save)
+                x = x.contiguous().float()
+                self.refresh_packs()
+                stem = self._pack_plan_cache[0]    # _packed_weights() lists the stem convolution first
+                if nc != stem.T:
+                    raise RuntimeError(f"{name}: expected {stem.T} input channels, got {nc}")
+                self._saving = bool(save)
+                patches = self.new(N, H, W, stem.K, x.device)
+                call("rbu_stem_im2col", _p(x), N, nc, H, W, stem.K, _vp(patches), stream_ptr())
+                # handed over inside S so that the body holds the only reference: inference frees the patches as soon as
+                # the first block has run
+                S = {"N": N, "H": H, "W": W, "patches": patches}
+                del patches
+                out = self._network_forward(S, training, save)
+                return out, (S if save else None)
         finally:
             self.flush_counters()
 
-    def _forward_impl(self, x: torch.Tensor, training: bool, save: bool):
+    def backward(self, S, dout: torch.Tensor, allreduce_hook=None):
+        """Returns {param_name: fp32 gradient} from the state of forward(..., save=True) and d(output).  A network may call
+        `allreduce_hook(names, grads, event)` as soon as the gradients of a top-level child are complete (reverse
+        execution order) so data-parallel buckets can overlap.  The network-specific part is _network_backward."""
+        with torch.cuda.device(dout.device):
+            grads = self._network_backward(S, dout, allreduce_hook)
+            self.join_side(dout.device)
+        return grads
+
+    def _network_forward(self, S, training: bool, save: bool):
+        """RobustUNet.forward (Main_Final.py:290-321) from the stem patches (S["patches"], taken out of S) to the
+        probabilities; fills S with the backward state when `save`."""
         m = self.model
-        _lib.check(0)
-        if not x.is_cuda:
-            raise RuntimeError("rbunet.RobustUNet runs on CUDA tensors only (no CPU fallback)")
-        N, nc, H, W = x.shape
-        if H % 16 or W % 16:
-            raise RuntimeError(f"input H,W must be multiples of 16, got {H}x{W}")
-        if nc != m.inc.conv1.in_channels:
-            raise RuntimeError(f"expected {m.inc.conv1.in_channels} input channels, got {nc}")
-        dev = x.device
-        x = x.contiguous().float()
-        self.refresh_packs()
-        self._saving = bool(save)
-        S = {"N": N, "H": H, "W": W}
-        Kp = ((9 * nc + 7) // 8) * 8
-        patches = View(torch.empty((N, H, W, Kp), dtype=torch.bfloat16, device=dev))
-        call("rbu_stem_im2col", _p(x), N, nc, H, W, Kp, _vp(patches), stream_ptr())
+        N, H, W = S["N"], S["H"], S["W"]
+        patches = S.pop("patches")
+        dev = patches.base.device
         enc = []
 
         def keep(key, st):          # inference: intermediates are released as soon as their block has run
@@ -770,9 +763,7 @@ class Engine:
             C = up.out_channels
             skip = enc[k - 1]
             cat = self.new(N, 2 * h, 2 * w, 2 * C, dev)
-            conv_gemm(N, h, w, [(cur, self.pack(up.weight, 2), 1, 0, False)], 4 * C, cat.slice(C, C), scatter=True,
-                      Cout=C, bias=up.bias)
-            keep(f"up{k}", {"x": cur, "N": N, "H": h, "W": w, "C": C})
+            keep(f"up{k}", self.up_forward(up, cur, N, h, w, cat.slice(C, C)))
             h, w = 2 * h, 2 * w
             st = self.ag_forward(getattr(m, f"att{k}"), cat.slice(C, C), skip, cat.slice(0, C), N, h, w, training)
             keep(f"att{k}", st)
@@ -795,15 +786,9 @@ class Engine:
         self.last_logits = logits
         S["head_x"] = cur
         S["probs"] = probs
-        return probs, (S if save else None)
+        return probs
 
-    def backward(self, S, dprobs: torch.Tensor, allreduce_hook=None):
-        """Returns {param_name: fp32 gradient}.  `allreduce_hook(names, grads)` is called as soon as the gradients
-        of a top-level child are complete (reverse execution order) so data-parallel buckets can overlap."""
-        with torch.cuda.device(dprobs.device):
-            return self._backward_impl(S, dprobs, allreduce_hook)
-
-    def _backward_impl(self, S, dprobs: torch.Tensor, allreduce_hook=None):
+    def _network_backward(self, S, dprobs: torch.Tensor, allreduce_hook):
         m = self.model
         grads = {}
         N, H, W = S["N"], S["H"], S["W"]
@@ -838,21 +823,10 @@ class Engine:
             sd = S[f"dec{k}"]
             dcat = self.rb_backward(getattr(m, f"dec{k}"), sd, d, grads, f"dec{k}")
             C = sd["C"]
-            hk, wk = sd["H"], sd["W"]
-            denc[k - 1] = self.new(N, hk, wk, C, dev)
+            denc[k - 1] = self.new(N, sd["H"], sd["W"], C, dev)
             self.ag_backward(getattr(m, f"att{k}"), S[f"att{k}"], dcat.slice(0, C), denc[k - 1], dcat.slice(C, C), grads,
                              f"att{k}")
-            up = getattr(m, f"up{k}")
-            su = S[f"up{k}"]
-            dup = dcat.slice(C, C)
-            gub = torch.empty_like(up.bias)
-            ws = self.bwd_ws(N, hk * wk, C, dev)
-            call("rbu_chan_sum", _vp(dup), dup.ld, N * hk * wk, C, _p(gub), _p(ws), ws.numel() * 4, stream_ptr())
-            d = self.new(N, su["H"], su["W"], su["x"].C, dev)
-            conv_gemm(N, su["H"], su["W"], [(dup, self.pack(up.weight, 3), 4, 0, True)], su["x"].C, d)
-            guw = self.gbuf(f"up{k}.weight", up.weight)
-            self.wgrad(N, su["H"], su["W"], su["x"], dup, 4, 0, True, guw)
-            grads[f"up{k}.bias"], grads[f"up{k}.weight"] = gub, guw
+            d = self.up_backward(getattr(m, f"up{k}"), S[f"up{k}"], dcat.slice(C, C), grads, f"up{k}")
             done(f"dec{k}", f"att{k}", f"up{k}")
         d = self.rb_backward(m.bottleneck[2], S["bott"], d, grads, "bottleneck.2")
         d = self.dil_backward(m.bottleneck[1], S["dil"], d, grads, "bottleneck.1")
@@ -871,5 +845,4 @@ class Engine:
             else:
                 self.rb_backward(m.inc, S["inc"], denc[0], grads, "inc", need_dx=False)
                 done("inc")
-        self.join_side(dev)
         return grads

@@ -201,9 +201,9 @@ class _Graph(torch.autograd.Function):
         model, state = ctx.model, ctx.state
         if state is None:
             raise RuntimeError(
-                "rbunet.RobustUNet: backward needs a train-mode forward with gradients enabled.  Backward through an "
-                "eval-mode forward (running-statistics BatchNorm) is not implemented: the backward kernels apply the "
-                "batch-statistics BatchNorm formulas of Main_Final.py:573-582's training loop and would return wrong "
+                f"rbunet.{type(model).__name__}: backward needs a train-mode forward with gradients enabled.  Backward "
+                "through an eval-mode forward (running-statistics BatchNorm) is not implemented: the backward kernels "
+                "apply the batch-statistics BatchNorm formulas of the reference's training loop and would return wrong "
                 "gradients, so this raises instead")
         ctx.state = None
         if model._grad_begin_hook is not None:
@@ -218,44 +218,16 @@ class _Graph(torch.autograd.Function):
         return (None, None, None, *out)
 
 
-class RobustUNet(nn.Module):
-    """B200-native Robust U-Net; same public surface as Main_Final.RobustUNet (Main_Final.py:226-321)."""
+class _Network(nn.Module):
+    """What RobustUNet and UNet share: forward() runs the whole network as one autograd node (_Graph) on the kernel
+    schedule of `engine_class(self)`."""
 
-    def __init__(self, n_channels=3, n_classes=1, base_channels=64):
+    def __init__(self, engine_class):
         super().__init__()
-        if not 1 <= n_classes <= 32:
-            raise ValueError(f"n_classes must be in [1, 32], got {n_classes}")
-        b = base_channels
-        if b < 16 or b & (b - 1):
-            raise ValueError("base_channels must be a power of two >= 16")
-        if n_classes > 1 and b > 256:
-            raise ValueError("the K-class head takes at most 256 input channels: base_channels <= 256 when n_classes > 1")
-        self.inc = ResidualBlock(n_channels, b, 0.1)
-        self.down1 = nn.Sequential(_Slot(), ResidualBlock(b, 2 * b, 0.1))
-        self.down2 = nn.Sequential(_Slot(), ResidualBlock(2 * b, 4 * b, 0.2))
-        self.down3 = nn.Sequential(_Slot(), ResidualBlock(4 * b, 8 * b, 0.2))
-        self.bottleneck = nn.Sequential(_Slot(), DilatedBlock(8 * b, 16 * b), ResidualBlock(16 * b, 16 * b, 0.3))
-        for k, c in ((4, 8 * b), (3, 4 * b), (2, 2 * b), (1, b)):
-            setattr(self, f"att{k}", AttentionGate(c, c, c // 2))
-        for k, c, p in ((4, 8 * b, 0.2), (3, 4 * b, 0.2), (2, 2 * b, 0.1), (1, b, 0.1)):
-            setattr(self, f"up{k}", nn.ConvTranspose2d(2 * c, c, 2, stride=2))
-            setattr(self, f"dec{k}", ResidualBlock(2 * c, c, p))
-        self.outc = nn.Sequential(nn.Conv2d(b, n_classes, 1), _Slot())
-        self._initialize_weights()
-        self._engine = Engine(self)
+        self._engine = engine_class(self)
         self._grad_begin_hook = None      # set by parallel.DataParallel: called with the engine when a backward starts
         self._grad_ready_hook = None      # set by parallel.DataParallel: called with the names of finished grads
         self._grad_transform = None       # set by parallel.DataParallel: swaps in the all-reduced gradients
-
-    def _initialize_weights(self):
-        """Kaiming-normal(fan_out, relu) on every Conv2d weight, BN gamma = 1 / beta = 0; ConvTranspose2d and all
-        biases keep torch's defaults (Main_Final.py:281-288)."""
-        for m in self.modules():
-            if isinstance(m, nn.Conv2d):
-                nn.init.kaiming_normal_(m.weight, mode="fan_out", nonlinearity="relu")
-            elif isinstance(m, nn.BatchNorm2d):
-                nn.init.ones_(m.weight)
-                nn.init.zeros_(m.bias)
 
     @property
     def engine(self) -> Engine:
@@ -290,9 +262,45 @@ class RobustUNet(nn.Module):
     def forward(self, x):
         params = tuple(p for _, p in self._named_params())
         if torch.is_grad_enabled() and x.requires_grad:
-            raise RuntimeError("rbunet.RobustUNet does not produce a gradient for its input (the first layer's data "
-                               "gradient is never computed); detach the input")
+            raise RuntimeError(f"rbunet.{type(self).__name__} does not produce a gradient for its input (the first "
+                               "layer's data gradient is never computed); detach the input")
         # grad mode is off inside autograd.Function.forward, so decide here whether to keep the backward state.  Only a
         # train-mode forward keeps it: the backward kernels implement batch-statistics BatchNorm (see _Graph.backward)
         save = self.training and torch.is_grad_enabled() and any(p.requires_grad for p in params)
         return _Graph.apply(self, save, x, *params)
+
+
+class RobustUNet(_Network):
+    """B200-native Robust U-Net; same public surface as Main_Final.RobustUNet (Main_Final.py:226-321)."""
+
+    def __init__(self, n_channels=3, n_classes=1, base_channels=64):
+        super().__init__(Engine)
+        if not 1 <= n_classes <= 32:
+            raise ValueError(f"n_classes must be in [1, 32], got {n_classes}")
+        b = base_channels
+        if b < 16 or b & (b - 1):
+            raise ValueError("base_channels must be a power of two >= 16")
+        if n_classes > 1 and b > 256:
+            raise ValueError("the K-class head takes at most 256 input channels: base_channels <= 256 when n_classes > 1")
+        self.inc = ResidualBlock(n_channels, b, 0.1)
+        self.down1 = nn.Sequential(_Slot(), ResidualBlock(b, 2 * b, 0.1))
+        self.down2 = nn.Sequential(_Slot(), ResidualBlock(2 * b, 4 * b, 0.2))
+        self.down3 = nn.Sequential(_Slot(), ResidualBlock(4 * b, 8 * b, 0.2))
+        self.bottleneck = nn.Sequential(_Slot(), DilatedBlock(8 * b, 16 * b), ResidualBlock(16 * b, 16 * b, 0.3))
+        for k, c in ((4, 8 * b), (3, 4 * b), (2, 2 * b), (1, b)):
+            setattr(self, f"att{k}", AttentionGate(c, c, c // 2))
+        for k, c, p in ((4, 8 * b, 0.2), (3, 4 * b, 0.2), (2, 2 * b, 0.1), (1, b, 0.1)):
+            setattr(self, f"up{k}", nn.ConvTranspose2d(2 * c, c, 2, stride=2))
+            setattr(self, f"dec{k}", ResidualBlock(2 * c, c, p))
+        self.outc = nn.Sequential(nn.Conv2d(b, n_classes, 1), _Slot())
+        self._initialize_weights()
+
+    def _initialize_weights(self):
+        """Kaiming-normal(fan_out, relu) on every Conv2d weight, BN gamma = 1 / beta = 0; ConvTranspose2d and all
+        biases keep torch's defaults (Main_Final.py:281-288)."""
+        for m in self.modules():
+            if isinstance(m, nn.Conv2d):
+                nn.init.kaiming_normal_(m.weight, mode="fan_out", nonlinearity="relu")
+            elif isinstance(m, nn.BatchNorm2d):
+                nn.init.ones_(m.weight)
+                nn.init.zeros_(m.bias)

@@ -43,20 +43,30 @@ def _p(t):
     return c_void_p(t.data_ptr()) if t is not None else c_void_p(0)
 
 
-def pack_weight(w: torch.Tensor, mode: int) -> torch.Tensor:
-    """fp32 torch-layout weight -> bf16 GEMM operand [Ncols][taps][K] (see rbu_pack_weight)."""
-    assert w.is_cuda and w.dtype == torch.float32 and w.is_contiguous()
+def pack_dims(w: torch.Tensor, mode: int):
+    """(Nn, T, K, Cout, destination shape) of the bf16 GEMM operand that rbu_pack_weight / rbu_pack_weights_multi build
+    from the fp32 torch-layout weight `w` in pack mode `mode`."""
     if mode == 0:            # Conv2d [Cout,Cin,kh,kw] forward
-        Nn, K, T, cout = w.shape[0], w.shape[1], w.shape[2] * w.shape[3], 0
+        Nn, T, K, cout = w.shape[0], w.shape[2] * w.shape[3], w.shape[1], 0
     elif mode == 1:          # Conv2d data gradient
-        Nn, K, T, cout = w.shape[1], w.shape[0], w.shape[2] * w.shape[3], 0
+        Nn, T, K, cout = w.shape[1], w.shape[2] * w.shape[3], w.shape[0], 0
     elif mode == 2:          # ConvTranspose2d [Cin,Cout,2,2] forward
-        Nn, K, T, cout = 4 * w.shape[1], w.shape[0], 1, w.shape[1]
+        Nn, T, K, cout = 4 * w.shape[1], 1, w.shape[0], w.shape[1]
     elif mode == 3:          # ConvTranspose2d data gradient
-        Nn, K, T, cout = w.shape[0], w.shape[1], 4, 0
+        Nn, T, K, cout = w.shape[0], 4, w.shape[1], 0
+    elif mode in (4, 5):     # stem Conv2d [C,nc,3,3] on the rbu_stem_im2col patches: [Nn][1][Kp] with T = nc; mode 4
+        nc = w.shape[1]      # also holds the 1x1 shortcut (second source) in rows C..2C-1
+        Nn, T, K, cout = (2 if mode == 4 else 1) * w.shape[0], nc, (9 * nc + 7) // 8 * 8, 0
     else:
         raise ValueError(mode)
-    out = torch.empty((Nn, T, K), dtype=torch.bfloat16, device=w.device)
+    return Nn, T, K, cout, ((Nn, 1, K) if mode >= 4 else (Nn, T, K))
+
+
+def pack_weight(w: torch.Tensor, mode: int) -> torch.Tensor:
+    """fp32 torch-layout weight -> bf16 GEMM operand [Ncols][taps][K] (see rbu_pack_weight; modes 0-3)."""
+    assert w.is_cuda and w.dtype == torch.float32 and w.is_contiguous()
+    Nn, T, K, cout, shape = pack_dims(w, mode)
+    out = torch.empty(shape, dtype=torch.bfloat16, device=w.device)
     call("rbu_pack_weight", _p(w), _p(out), Nn, T, K, mode, cout, stream_ptr())
     return out
 

@@ -18,7 +18,7 @@ import torch.nn as nn
 from . import _lib
 from ._lib import call, stream_ptr
 from .engine import NULL, Engine, _p, _vp
-from .model import _Slot
+from .model import _Network, _Slot
 from .ops import View, conv_gemm
 
 
@@ -26,33 +26,13 @@ class UNetEngine(Engine):
     LEVELS = ((1, 64), (2, 128), (3, 256), (4, 512))
 
     # ------------------------------------------------------------------ weight operands
-    def _pack_plan(self):
+    def _packed_weights(self):
         m = self.model
-        jobs = []
-
-        def conv(w, mode):
-            if mode == 0:
-                Nn, K, T = w.shape[0], w.shape[1], 9
-            else:
-                Nn, K, T = w.shape[1], w.shape[0], 9
-            jobs.append(((id(w), mode), w, None, (Nn, T, K), Nn, T, K, mode, 0))
-
-        w0 = m.enc1[0].weight
-        nc = w0.shape[1]
-        Kp = ((9 * nc + 7) // 8) * 8
-        jobs.append(((id(w0), "stem"), w0, None, (w0.shape[0], 1, Kp), w0.shape[0], nc, Kp, 5, 0))
-        for name in ("enc1", "enc2", "enc3", "enc4", "bottleneck", "dec4", "dec3", "dec2", "dec1"):
+        out = [(m.enc1[0].weight, (5,)), (m.enc1[3].weight, (0, 1))]
+        for name in ("enc2", "enc3", "enc4", "bottleneck", "dec4", "dec3", "dec2", "dec1"):
             seq = getattr(m, name)
-            if name != "enc1":
-                conv(seq[0].weight, 0)
-                conv(seq[0].weight, 1)
-            conv(seq[3].weight, 0)
-            conv(seq[3].weight, 1)
-        for k in (4, 3, 2, 1):
-            w = getattr(m, f"upconv{k}").weight
-            jobs.append(((id(w), 2), w, None, (4 * w.shape[1], 1, w.shape[0]), 4 * w.shape[1], 1, w.shape[0], 2, w.shape[1]))
-            jobs.append(((id(w), 3), w, None, (w.shape[0], 4, w.shape[1]), w.shape[0], 4, w.shape[1], 3, 0))
-        return jobs
+            out += [(seq[0].weight, (0, 1)), (seq[3].weight, (0, 1))]
+        return out + [(getattr(m, f"upconv{k}").weight, (2, 3)) for k in (4, 3, 2, 1)]
 
     # ------------------------------------------------------------------ conv_block (train_water_segmentation.py:251-260)
     def block_forward(self, seq, x: View, N, H, W, training, out: View = None, patches: View = None):
@@ -66,7 +46,7 @@ class UNetEngine(Engine):
             f1 = self.bn_eval_affine(seq[1], src, seq[0].bias)
             a1 = self.new(N, H, W, C, dev)
             if patches is not None:
-                conv_gemm(N, H, W, [(patches, self._packs[(id(seq[0].weight), "stem")], 1, 0, False)], C, a1,
+                conv_gemm(N, H, W, [(patches, self._packs[(id(seq[0].weight), 5)], 1, 0, False)], C, a1,
                           scale=f1["scale"], bias=f1["shift"], relu=C, flops=2.0 * P * C * 9 * seq[0].in_channels)
             else:
                 conv_gemm(N, H, W, [(x, self.pack(seq[0].weight, 0), 9, 1, False)], C, a1, scale=f1["scale"],
@@ -79,7 +59,7 @@ class UNetEngine(Engine):
             return out, None
         y1 = self.new(N, H, W, C, dev)
         if patches is not None:
-            conv_gemm(N, H, W, [(patches, self._packs[(id(seq[0].weight), "stem")], 1, 0, False)], C, y1, bias=seq[0].bias,
+            conv_gemm(N, H, W, [(patches, self._packs[(id(seq[0].weight), 5)], 1, 0, False)], C, y1, bias=seq[0].bias,
                       flops=2.0 * P * C * 9 * seq[0].in_channels)
         else:
             conv_gemm(N, H, W, [(x, self.pack(seq[0].weight, 0), 9, 1, False)], C, y1, bias=seq[0].bias)
@@ -139,23 +119,11 @@ class UNetEngine(Engine):
         return dx
 
     # ------------------------------------------------------------------ whole model (:262-288)
-    def _forward_impl(self, x: torch.Tensor, training: bool, save: bool):
+    def _network_forward(self, S, training: bool, save: bool):
         m = self.model
-        if not x.is_cuda:
-            raise RuntimeError("rbunet.UNet runs on CUDA tensors only (no CPU fallback)")
-        N, nc, H, W = x.shape
-        if H % 16 or W % 16:
-            raise RuntimeError(f"input H,W must be multiples of 16, got {H}x{W}")
-        if nc != m.enc1[0].in_channels:
-            raise RuntimeError(f"expected {m.enc1[0].in_channels} input channels, got {nc}")
-        dev = x.device
-        x = x.contiguous().float()
-        self.refresh_packs()
-        self._saving = bool(save)
-        S = {"N": N, "H": H, "W": W}
-        Kp = ((9 * nc + 7) // 8) * 8
-        patches = View(torch.empty((N, H, W, Kp), dtype=torch.bfloat16, device=dev))
-        call("rbu_stem_im2col", _p(x), N, nc, H, W, Kp, _vp(patches), stream_ptr())
+        N, H, W = S["N"], S["H"], S["W"]
+        patches = S.pop("patches")
+        dev = patches.base.device
         cats, h, w = {}, H, W
         cur = None
         for lvl, C in self.LEVELS:                     # encoder output k lives in the second half of concat buffer k
@@ -175,12 +143,10 @@ class UNetEngine(Engine):
         if save:
             S["bottleneck"] = st
         for lvl, C in reversed(self.LEVELS):
-            up = getattr(m, f"upconv{lvl}")
             cat = cats[lvl]
-            conv_gemm(N, h, w, [(cur, self.pack(up.weight, 2), 1, 0, False)], 4 * C, cat.slice(0, C), scatter=True, Cout=C,
-                      bias=up.bias)
+            st = self.up_forward(getattr(m, f"upconv{lvl}"), cur, N, h, w, cat.slice(0, C))
             if save:
-                S[f"up{lvl}"] = {"x": cur, "H": h, "W": w, "C": C}
+                S[f"up{lvl}"] = st
             h, w = 2 * h, 2 * w
             cur, st = self.block_forward(getattr(m, f"dec{lvl}"), cat, N, h, w, training)
             if save:
@@ -199,9 +165,9 @@ class UNetEngine(Engine):
         if save:
             S["cats"] = cats
             S["head_x"] = cur
-        return logits, (S if save else None)
+        return logits
 
-    def backward(self, S, dlogits: torch.Tensor, allreduce_hook=None):
+    def _network_backward(self, S, dlogits: torch.Tensor, allreduce_hook):
         m = self.model
         grads = {}
         N, H, W = S["N"], S["H"], S["W"]
@@ -223,19 +189,8 @@ class UNetEngine(Engine):
         denc = {}
         for lvl, C in self.LEVELS:
             dcat = self.block_backward(getattr(m, f"dec{lvl}"), S[f"dec{lvl}"], d, grads, f"dec{lvl}")
-            su = S[f"up{lvl}"]
-            up = getattr(m, f"upconv{lvl}")
-            dup = dcat.slice(0, C)
             denc[lvl] = dcat.slice(C, C)
-            hk, wk = 2 * su["H"], 2 * su["W"]
-            gub = torch.empty_like(up.bias)
-            ws = self.bwd_ws(N, hk * wk, C, dev)
-            call("rbu_chan_sum", _vp(dup), dup.ld, N * hk * wk, C, _p(gub), _p(ws), ws.numel() * 4, stream_ptr())
-            guw = torch.empty_like(up.weight)
-            self.wgrad(N, su["H"], su["W"], su["x"], dup, 4, 0, True, guw)
-            grads[f"upconv{lvl}.bias"], grads[f"upconv{lvl}.weight"] = gub, guw
-            d = self.new(N, su["H"], su["W"], su["x"].C, dev)
-            conv_gemm(N, su["H"], su["W"], [(dup, self.pack(up.weight, 3), 4, 0, True)], su["x"].C, d)
+            d = self.up_backward(getattr(m, f"upconv{lvl}"), S[f"up{lvl}"], dcat.slice(0, C), grads, f"upconv{lvl}")
         d = self.block_backward(m.bottleneck, S["bottleneck"], d, grads, "bottleneck")
         cats = S["cats"]
         for lvl, C in reversed(self.LEVELS):
@@ -244,30 +199,7 @@ class UNetEngine(Engine):
             call("rbu_maxpool2x2_bwd", _vp(src), src.ld, _vp(d), d.ld, _vp(denc[lvl]), denc[lvl].ld, N, ho, wo, C, 1,
                  stream_ptr())
             d = self.block_backward(getattr(m, f"enc{lvl}"), S[f"enc{lvl}"], denc[lvl], grads, f"enc{lvl}", need_dx=lvl > 1)
-        self.join_side(dev)
         return grads
-
-
-class _UNetGraph(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, model, save, x, *params):
-        logits, state = model._engine.forward(x, model.training, save)
-        ctx.model = model
-        ctx.state = state
-        return logits
-
-    @staticmethod
-    def backward(ctx, dlogits):
-        model, state = ctx.model, ctx.state
-        if state is None:
-            raise RuntimeError("backward through rbunet.UNet without a saved forward state")
-        ctx.state = None
-        grads = model._engine.backward(state, dlogits)
-        out = []
-        for name, p in model.named_parameters():
-            g = grads.get(name) if p.requires_grad else None
-            out.append(g.reshape(p.shape) if g is not None else None)
-        return (None, None, None, *out)
 
 
 def _conv_block(ci, co):
@@ -275,11 +207,11 @@ def _conv_block(ci, co):
                          nn.Conv2d(co, co, 3, padding=1), nn.BatchNorm2d(co), _Slot())
 
 
-class UNet(nn.Module):
+class UNet(_Network):
     """B200-native plain U-Net; same public surface as train_water_segmentation.UNet (:209-288)."""
 
     def __init__(self, n_channels=3, n_classes=2):
-        super().__init__()
+        super().__init__(UNetEngine)
         if not 1 <= n_classes <= 32:
             raise ValueError(f"n_classes must be in [1, 32], got {n_classes}")
         self.enc1 = _conv_block(n_channels, 64)
@@ -292,16 +224,6 @@ class UNet(nn.Module):
             setattr(self, f"dec{k}", _conv_block(2 * c, c))
         self.final = nn.Conv2d(64, n_classes, kernel_size=1)
         self.pool = _Slot()
-        self._engine = UNetEngine(self)
-
-    @property
-    def engine(self):
-        return self._engine
-
-    def forward(self, x):
-        params = tuple(self.parameters())
-        save = torch.is_grad_enabled() and any(p.requires_grad for p in params)
-        return _UNetGraph.apply(self, save, x, *params)
 
 
 class _CE2(torch.autograd.Function):

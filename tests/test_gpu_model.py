@@ -221,6 +221,44 @@ def test_weights_are_repacked_after_a_fused_optimizer_step():
     assert rel_l2(p1, pref) < 5e-2                              # and it is the update the masters hold
 
 
+@pytest.mark.parametrize("net", ["RobustUNet", "UNet"])
+def test_pack_plan_is_built_once_per_set_of_parameters(net):
+    """The weight-pack job list is reused while the modules hold the same Parameter objects (in-place optimizer steps);
+    load_state_dict(assign=True) replaces them and rebuilds it once, and equal values give bit-identical outputs."""
+    import rbunet
+    dev = torch.device("cuda:0")
+    torch.manual_seed(0)
+    x, y = R.synthetic_inputs(2, 3, 32, 32, seed=5, blobby=True)
+    if net == "UNet":
+        model, crit, y = rbunet.UNet(3, 2), rbunet.CrossEntropyArgmaxLoss(), y[:, 0].long()
+    else:
+        model, crit = rbunet.RobustUNet(3, 1, 16), rbunet.RobustBCEDiceLoss()
+    model.to(dev).train()
+    x, y = x.to(dev), y.to(dev)
+    eng, builds = model.engine, []
+    build = eng._pack_plan
+
+    def counted():
+        builds.append(1)
+        return build()
+
+    eng._pack_plan = counted
+    opt = torch.optim.SGD(model.parameters(), lr=1e-3)
+    for _ in range(3):
+        opt.zero_grad()
+        crit(model(x), y).backward()
+        opt.step()
+    assert len(builds) == 1
+    model.eval()
+    with torch.no_grad():
+        before = model(x).clone()
+    model.load_state_dict({k: v.clone() for k, v in model.state_dict().items()}, assign=True)
+    with torch.no_grad():
+        after = model(x)
+    assert len(builds) == 2
+    assert torch.equal(before, after)
+
+
 @pytest.mark.parametrize("B,H,W", [(1, 16, 16), (3, 16, 32), (1, 48, 16)])
 def test_minimum_and_ragged_input_sizes(B, H, W):
     """Smallest legal inputs (H, W multiples of 16: the bottleneck sees 1 x 1 and 1 x 2 pixels, below every halo-kernel

@@ -90,10 +90,23 @@ def test_gradients_have_private_storage_clip_and_accumulate():
 
 def test_eval_mode_backward_raises_instead_of_returning_wrong_gradients():
     import rbunet
+    _check_eval_mode_backward_raises(rbunet.RobustUNet(3, 1, 16), rbunet.RobustBCEDiceLoss(), lambda y: y)
+
+
+def test_unet_eval_mode_backward_raises_instead_of_returning_wrong_gradients():
+    import rbunet
+    _check_eval_mode_backward_raises(rbunet.UNet(3, 2), rbunet.CrossEntropyArgmaxLoss(), lambda y: y[:, 0].long())
+
+
+def _check_eval_mode_backward_raises(model, crit, target):
     dev = torch.device("cuda:0")
-    model = rbunet.RobustUNet(3, 1, 16).to(dev).eval()
     x, y = R.synthetic_inputs(1, 3, 32, 32, seed=3, blobby=True)
-    loss = rbunet.RobustBCEDiceLoss()(model(x.to(dev)), y.to(dev))       # forward in eval mode with grad enabled works
+    y = target(y)
+    model.to(dev).eval()
+    out = model(x.to(dev))                                  # forward in eval mode with grad enabled works
+    with torch.no_grad():
+        assert torch.equal(out, model(x.to(dev)))           # and computes what it computes without grad
+    loss = crit(out, y.to(dev))
     with pytest.raises(RuntimeError, match="train-mode forward"):
         loss.backward()
     with pytest.raises(RuntimeError, match="gradient for its input"):
