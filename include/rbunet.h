@@ -352,6 +352,26 @@ int rbu_cek_forward(const float* logits, const int64_t* target, int B, int64_t H
 int rbu_cek_backward(const float* logits, const int64_t* target, int B, int64_t HW, int K, const float* grad_out,
                      float* dlogits, void* stream);
 
+/* ------------------------------------------------------------------ tiled whole-scene inference
+ * Sliding-window prediction at full resolution, the alternative to predict_coastline.py:386-392,583-602 (resize the
+ * scene to 512², predict, scale the mask back up).  The tile grid is ny x nx tiles of th x tw; tile t = iy*nx + ix has
+ * its origin at (oy[iy], ox[ix]) (DEVICE int tables).  Tile rows / columns beyond the scene are reflected with
+ * F.pad(mode="reflect") semantics, so th <= 2H - 1 and tw <= 2W - 1.
+ *
+ * rbu_tile_gather: x fp32 NCHW [nc,H,W] -> out fp32 [Tb][nc][th][tw], tiles t0 .. t0+Tb-1. */
+int rbu_tile_gather(const float* x, int nc, int H, int W, const int* oy, const int* ox, int ny, int nx, int th, int tw,
+                    int t0, int Tb, float* out, void* stream);
+/* rbu_tile_blend: tiles fp32 [ny*nx][K][th][tw] (1 <= K <= 32) -> labels uint8 [H,W] and, when out != NULL, the blended
+ * fp32 [K][H][W].  Output row y is covered by tiles iy in [row_first[y], row_first[y] + row_count[y]), column x by
+ * ix in [col_first[x], col_first[x] + col_count[x]) (DEVICE int tables); wy [th] / wx [tw] are the 1-D window weights.
+ * Per pixel, over iy ascending (outer) and ix ascending (inner), each a separately rounded fp32 operation:
+ *   w = wy[y - oy[iy]] * wx[x - ox[ix]];  num_k += w * v_k;  den += w;   out_k = num_k / den.
+ * labels = out_0 > threshold (strict) at K = 1, else the arg-max over k (ties -> lowest k, as torch.argmax).  A gather
+ * with no atomics: bit-deterministic. */
+int rbu_tile_blend(const float* tiles, int K, int H, int W, const int* oy, const int* ox, int ny, int nx, int th, int tw,
+                   const int* row_first, const int* row_count, const int* col_first, const int* col_count,
+                   const float* wy, const float* wx, float threshold, float* out, uint8_t* labels, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
