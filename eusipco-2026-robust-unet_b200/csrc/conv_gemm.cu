@@ -594,6 +594,9 @@ extern "C" int rbu_conv_gemm(const rbu_conv_gemm_args* a, void* stream_) {
                   "rbu_conv_gemm: scatter needs Ncols == 4*Cout and Cout %% 8 == 0");
     RBU_CHECK_ARG(a->addend == nullptr, "rbu_conv_gemm: addend is not supported with scatter");
   }
+  // both epilogues rectify whole 8-channel groups (cb < relu per group), so only a multiple of 8 names a channel prefix
+  RBU_CHECK_ARG(a->relu >= 0 && a->relu % 8 == 0 && a->relu <= (a->scatter ? a->Cout : a->Ncols),
+                "rbu_conv_gemm: relu=%d must be a multiple of 8 in [0, %d]", a->relu, a->scatter ? a->Cout : a->Ncols);
   if (a->addend)
     RBU_CHECK_ARG(a->addend_ld % 8 == 0 && ((uintptr_t)a->addend & 15) == 0, "rbu_conv_gemm: addend view misaligned");
   int gather = 0;

@@ -31,7 +31,7 @@ struct WParams {
   int TW, TH, TN;
   int tiles_w, tiles_h, tiles_n, tiles_total;
   int Mtot, Ntot, taps, dil, gather;
-  int tap_first, tap_end;        // taps [tap_first, tap_end) are computed (all of them, or tap 8 for the halo kernel)
+  int tap_first, tap_end;        // taps [tap_first, tap_end) are computed (rbu_wgrad_gemm: all of them)
   int BM, BN, T;                 // block sizes; T taps per work item
   int m_blocks, n_blocks, t_groups, ksplit, items;
   int b_stages, tmem_cols;
@@ -388,8 +388,8 @@ extern "C" size_t rbu_wgrad_workspace_bytes(const rbu_wgrad_args* a) {
   return pl.ws_bytes;
 }
 
-// The generic kernel restricted to taps [tap_first, tap_end) (tap_end < 0: all).  Used directly by rbu_wgrad_gemm and, for
-// tap 8 of a 3x3 convolution, by the halo kernel's 128-output-channel variant.
+// The generic kernel restricted to taps [tap_first, tap_end) (tap_end < 0: all).  Its only caller, rbu_wgrad_gemm, passes
+// the whole tap range; the halo kernels (wgrad_halo.cu) compute all nine taps themselves and never call this.
 size_t rbu_wgrad_generic_workspace_bytes(const rbu_wgrad_args* a, int tap_first, int tap_end) {
   Plan pl;
   make_plan(a, &pl, tap_first, tap_end);

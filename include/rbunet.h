@@ -107,7 +107,9 @@ typedef struct {
   const void* addend;       /* optional bf16 NHWC view added to the result (scatter=0 only)        */
   int64_t addend_ld;
   const float* scale;       /* optional fp32 [Cout]: y = scale*acc + bias (eval-mode BatchNorm folded into the conv) */
-  int relu;                 /* ReLU after scale / bias / addend on output channels [0, relu) (0: none)         */
+  int relu;                 /* ReLU after scale / bias / addend on output channels [0, relu) (0: none);        */
+                            /* a multiple of 8 (the epilogue works on 8-channel groups), at most Ncols (Cout   */
+                            /* when scatter=1); anything else is RBU_ERR_INVALID                               */
   float* stats;             /* optional: rbu_conv_stats_floats(Ncols) floats receiving one row per CTA of      */
                             /* partial sum / sum of squares per output column of the STORED (bf16) result --  */
                             /* the BatchNorm batch statistics, fused into the epilogue (scatter=0 only)        */
