@@ -6,6 +6,7 @@ Drop-in surface (reference: /root/reference/Main_Final.py):
   RobustBCEDiceLoss()  (defaults == nn.BCELoss())           Main_Final.py:551,580
   calculate_metrics(pred, target, threshold=0.5)            Main_Final.py:519-547
   predict_tiled(model, scene, tile, overlap)                whole scene at full resolution (predict_coastline.py:386-392)
+  PatchSampler(images, masks, size, ...).sample(B)          training patches of whole scenes at native resolution
 Everything below that surface is hand-written CUDA in csrc/ reached through the C ABI of
 librbunet.so (include/rbunet.h).  There is no CPU fallback.
 """
@@ -16,8 +17,9 @@ from .model import AttentionGate, DilatedBlock, ResidualBlock, RobustUNet  # noq
 from .ops import View, coastline_mask, enhance_image, preprocess, resize  # noqa: F401
 from .optim import FusedAdam  # noqa: F401
 from .parallel import DataParallel, GradBucketer  # noqa: F401
+from .patches import PatchSampler  # noqa: F401
 from .tiled import predict_tiled  # noqa: F401
 from .unet import CrossEntropyArgmaxLoss, UNet  # noqa: F401
 
 __all__ = ["RobustUNet", "ResidualBlock", "AttentionGate", "DilatedBlock", "RobustBCEDiceLoss", "calculate_metrics", "batch_metrics", "confusion_counts", "class_confusion_counts", "class_metrics",
-           "metrics_from_counts", "METRIC_KEYS", "View", "preprocess", "resize", "enhance_image", "coastline_mask", "predict_tiled", "DataParallel", "GradBucketer", "FusedAdam", "UNet", "CrossEntropyArgmaxLoss"]
+           "metrics_from_counts", "METRIC_KEYS", "View", "preprocess", "resize", "enhance_image", "coastline_mask", "predict_tiled", "PatchSampler", "DataParallel", "GradBucketer", "FusedAdam", "UNet", "CrossEntropyArgmaxLoss"]

@@ -1,47 +1,16 @@
-// Input preprocessing: uint8 RGB [B,H,W,3] -> fp32 NCHW planes.  Channels 0-2 are torchvision's ToTensor + Normalize
-// with the ImageNet constants (Main_Final.py:697-701): (x/255 - mean)/std.  The reference has no HSV code
-// (SURVEY.md §8c): the optional extra planes are build-defined and pinned to OpenCV float semantics --
-// n_channels == 4 appends S; n_channels == 6 appends H/360, S, V.  Every operation is an explicitly rounded IEEE
-// fp32 op (no FMA contraction), so the result is bit-identical to the numpy oracle.
-#include "rbu_common.cuh"
+// Input preprocessing: uint8 RGB [B,H,W,3] -> fp32 NCHW planes, the arithmetic of preprocess_pixel (preprocess.cuh):
+// Normalize in channels 0-2, the build-defined HSV planes beyond, bit-identical to the numpy oracle.
+#include "preprocess.cuh"
 
 namespace {
 
 __global__ void __launch_bounds__(256)
 preprocess_kernel(const uint8_t* __restrict__ img, long P, int HW, int nc, float* __restrict__ out) {
-  const float mean[3] = {0.485f, 0.456f, 0.406f};
-  const float stdv[3] = {0.229f, 0.224f, 0.225f};
   for (long p = blockIdx.x * (long)blockDim.x + threadIdx.x; p < P; p += (long)gridDim.x * blockDim.x) {
     const long n = p / HW;
     const long pl = p - n * HW;
-    float c[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) c[k] = __fdiv_rn((float)img[p * 3 + k], 255.0f);
-    float* o = out + n * (long)nc * HW + pl;
-#pragma unroll
-    for (int k = 0; k < 3; ++k) o[(long)k * HW] = __fdiv_rn(__fsub_rn(c[k], mean[k]), stdv[k]);
-    if (nc > 3) {
-      const float r = c[0], g = c[1], b = c[2];
-      const float v = fmaxf(fmaxf(r, g), b);
-      const float mn = fminf(fminf(r, g), b);
-      const float diff = __fsub_rn(v, mn);
-      const float s = v > 0.f ? __fdiv_rn(diff, v) : 0.f;
-      if (nc == 4) {
-        o[3L * HW] = s;
-      } else {
-        float h = 0.f;
-        if (diff > 0.f) {
-          if (v == r) h = __fdiv_rn(__fsub_rn(g, b), diff);
-          else if (v == g) h = __fadd_rn(2.0f, __fdiv_rn(__fsub_rn(b, r), diff));
-          else h = __fadd_rn(4.0f, __fdiv_rn(__fsub_rn(r, g), diff));
-          h = __fmul_rn(h, 60.0f);
-          if (h < 0.f) h = __fadd_rn(h, 360.0f);
-        }
-        o[3L * HW] = __fdiv_rn(h, 360.0f);
-        o[4L * HW] = s;
-        o[5L * HW] = v;
-      }
-    }
+    const uint8_t rgb[3] = {img[p * 3], img[p * 3 + 1], img[p * 3 + 2]};
+    preprocess_pixel(rgb, nc, out + n * (long)nc * HW + pl, HW);
   }
 }
 

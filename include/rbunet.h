@@ -374,6 +374,36 @@ int rbu_tile_blend(const float* tiles, int K, int H, int W, const int* oy, const
                    const int* row_first, const int* row_count, const int* col_first, const int* col_count,
                    const float* wy, const float* wx, float threshold, float* out, uint8_t* labels, void* stream);
 
+/* ------------------------------------------------------------------ patch sampling for native-resolution training
+ * The training-side counterpart of the tiled inference above, instead of the reference's whole-image resize to 512²
+ * (Main_Final.py:44-54,697-701): random ph x pw crops of whole scenes under the eight flips / 90-degree rotations, a
+ * fraction of them centred on a focus pixel (nnU-Net's foreground oversampling, MONAI's RandCropByPosNegLabel).  One
+ * launch per call.  srcs_device: DEVICE array of S scene descriptors (pitches in bytes; the bytes of a row's pixels are
+ * contiguous); focus_rows[y] = number of nonzero focus pixels in rows [0, y) (int64 [H+1]).  jobs_device: DEVICE array of
+ * B jobs; job b writes patch b:
+ *  - op 0-7: bit 2 transposes, bit 1 flips rows, bit 0 flips columns, in that order (out = win; out = out.transpose(-2,-1)
+ *    if bit 2; out = out.flip(-2) if bit 1; out = out.flip(-1) if bit 0).  The window is ph x pw for ops 0-3 and pw x ph
+ *    for ops 4-7, so every patch is ph x pw: out[i][j] = win[a][b] with i' = bit1 ? ph-1-i : i, j' = bit0 ? pw-1-j : j and
+ *    (a, b) = bit2 ? (j', i') : (i', j').
+ *  - origin: (y0, x0), unless focus != 0 and the scene has focus pixels (focus and focus_rows non-NULL, focus_rows[H] > 0):
+ *    then with k = r mod focus_rows[H] (r read as unsigned) and (py, px) the k-th nonzero focus pixel in row-major order,
+ *    y = clamp(py - wh/2, 0, H - wh), x = clamp(px - ww/2, 0, W - ww) for the wh x ww window, so the patch holds (py, px).
+ *  - images_out: fp32 [B][n_channels][ph][pw], bit for bit rbu_preprocess of the transformed uint8 patch (n_channels 3,
+ *    4 or 6); masks_out: uint8 [B][ph][pw], the mask window under the same transform, raw values; jobs_out (optional):
+ *    int32 [B][4] = (scene, y, x, op) of the resolved origin.
+ *  A job whose scene index or op is out of range, whose window is larger than its scene or whose (y0, x0) does not fit
+ *  leaves its patch unwritten and gets (-1, -1, -1, -1) in jobs_out.  64-bit offsets: scenes may exceed 2 GiB. */
+typedef struct {
+  const uint8_t* image;  long long image_pitch;   /* [H][W][3] uint8 RGB                                  */
+  const uint8_t* mask;   long long mask_pitch;    /* [H][W] uint8, any values                             */
+  const uint8_t* focus;  long long focus_pitch;   /* [H][W] uint8, nonzero = focus pixel; NULL if none    */
+  const long long* focus_rows;                    /* [H+1] exclusive prefix of nonzero focus pixels per row */
+  int H, W;
+} rbu_patch_src;
+typedef struct { int scene, op, y0, x0, focus, pad; long long r; } rbu_patch_job;   /* 32 bytes */
+int rbu_sample_patches(const rbu_patch_src* srcs_device, int S, const rbu_patch_job* jobs_device, int B, int ph, int pw,
+                       int n_channels, float* images_out, uint8_t* masks_out, int* jobs_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
