@@ -19,7 +19,6 @@
 #include "rbu_ptx.cuh"
 #include "tma_host.cuh"
 #include "gemm_epilogue.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -614,11 +613,7 @@ extern "C" int rbu_conv_gemm(const rbu_conv_gemm_args* a, void* stream_) {
     }
   }
 
-  {
-    static int no_halo = -1;   // RBU_NO_HALO=1 forces the generic per-tap kernel (A/B comparisons in the tests)
-    if (no_halo < 0) no_halo = getenv("RBU_NO_HALO") ? 1 : 0;
-    if (!no_halo && rbu_conv_halo_supported(a)) return rbu_conv_halo_launch(a, stream);
-  }
+  if (rbu_conv_halo_supported(a)) return rbu_conv_halo_launch(a, stream);
   RBU_CHECK_ARG(a->tile_stats == nullptr, "rbu_conv_gemm: tile statistics are produced by the 3x3 halo kernel only");
 
   KParams p;
@@ -661,12 +656,10 @@ extern "C" int rbu_conv_gemm(const rbu_conv_gemm_args* a, void* stream_) {
   p.fd_cout = make_fastdiv(a->scatter ? a->Cout : a->Ncols);
   // Staged epilogue (TMA stores) whenever the output is expressible as 32-pixel x 32-channel boxes of a tensor map:
   // whole 32-column chunks, and for the ConvTranspose pixel shuffle a warp's 32 pixels must be whole rows of the
-  // merged (n, h) axis.  RBU_NO_TMA_STORE=1 forces the per-thread stores (A/B comparisons in the tests).
+  // merged (n, h) axis.
   {
-    static int no_tma_store = -1;
-    if (no_tma_store < 0) no_tma_store = getenv("RBU_NO_TMA_STORE") ? 1 : 0;
     const int rows = 32 / p.TW;   // rows of the h axis in one warp's box when it does not span images
-    bool ok = !no_tma_store && a->Ncols % 32 == 0 && (!a->stats || (!gather && !a->scatter));
+    bool ok = a->Ncols % 32 == 0 && (!a->stats || (!gather && !a->scatter));
     if (a->scatter)
       ok = ok && a->Cout % 64 == 0 && ((p.TW * p.TH >= 32 && a->H % rows == 0) || p.TH == a->H);
     p.tma_store = ok ? 1 : 0;
@@ -675,15 +668,11 @@ extern "C" int rbu_conv_gemm(const rbu_conv_gemm_args* a, void* stream_) {
   if (grid > rbu_num_sms()) grid = rbu_num_sms();
   // Weights resident in shared memory when the CTA's whole operand (its column block, all k-blocks) is at most 64 KB and
   // every tile of a CTA has the same column block: the small-K GEMMs are bound by L2 -> SM traffic, of which the per-tile
-  // weight reload is 17-40%.  RBU_NO_RESIDENT=1 disables.
+  // weight reload is 17-40%.
   int kblocks_total = 0;
   for (int s = 0; s < a->nseg; ++s) kblocks_total += a->seg[s].taps * rbu_cdiv(a->seg[s].C, BLOCK_K);
   const int resb_bytes = kblocks_total * p.block_n * 128;
-  {
-    static int no_res = -1;
-    if (no_res < 0) no_res = getenv("RBU_NO_RESIDENT") ? 1 : 0;
-    p.b_resident = (!no_res && resb_bytes <= 65536 && grid % p.n_blocks == 0) ? 1 : 0;
-  }
+  p.b_resident = (resb_bytes <= 65536 && grid % p.n_blocks == 0) ? 1 : 0;
   const int staging = 1024 + (p.tma_store ? 8 * ST_BUFS * STG_BYTES : 0) + (p.b_resident ? resb_bytes : 0);
   const int stage_bytes = A_BYTES + (p.b_resident ? 0 : p.block_n * 128);
   p.num_stages = (SMEM_LIMIT - 1024 - BAR_BYTES - staging) / stage_bytes;

@@ -31,7 +31,6 @@
 #include "rbu_ptx.cuh"
 #include "tma_host.cuh"
 #include "gemm_epilogue.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -688,16 +687,6 @@ conv_halo_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_con
   conv_halo_body<true>(tmA0, tmB0, tmA1, tmB1, tmY, p);
 }
 
-// debug switches, read once per process
-struct Switches {
-  int no_pair, force_pair, no_resident, no_tma_store;
-};
-const Switches& switches() {
-  static const Switches sw = {getenv("RBU_CONV_NOPAIR") ? 1 : 0, getenv("RBU_CONV_PAIR") ? 1 : 0,
-                              getenv("RBU_NO_RESIDENT") ? 1 : 0, getenv("RBU_NO_TMA_STORE") ? 1 : 0};
-  return sw;
-}
-
 }  // namespace
 
 // Returns 1 if the halo kernel can run these arguments (3x3 dilation-1 and 1x1 segments on images of at least
@@ -706,9 +695,7 @@ int rbu_conv_halo_supported(const rbu_conv_gemm_args* a) {
   if (a->scatter || a->H < TILE_H || a->W < TILE_W) return 0;
   // per-CTA statistics: register accumulators on the staged path (any width that is whole 32-column chunks), shared-memory
   // accumulators covering 128 columns on the per-thread path
-  if (a->stats && a->Ncols > 32 * EPI_STAT_CHUNKS &&
-      (a->Ncols % 32 != 0 || switches().no_tma_store || switches().no_pair))
-    return 0;
+  if (a->stats && a->Ncols > 32 * EPI_STAT_CHUNKS && a->Ncols % 32 != 0) return 0;
   int any3x3 = 0;
   for (int s = 0; s < a->nseg; ++s) {
     const rbu_gemm_operand& o = a->seg[s];
@@ -748,20 +735,17 @@ int rbu_conv_halo_launch(const rbu_conv_gemm_args* a, cudaStream_t stream) {
   // and make the 128->64 layer's weights resident (72 KB per CTA).  Not used where a single CTA already keeps the whole
   // weight operand resident (64->64: nothing left to halve, and the pair's lock step costs 10 %; measured 918 vs 1020
   // TFLOP/s), with the per-CTA output statistics (unused by the engine), or for column blocks whose halves are not whole
-  // 8-row swizzle groups.  RBU_CONV_NOPAIR=1 selects the single-CTA kernel everywhere (A/B runs), RBU_CONV_PAIR=1 the
-  // pair kernel wherever it can run.
-  const int pair_mode = switches().no_pair ? 0 : (switches().force_pair ? 2 : 1);     // 0 never, 1 by shape, 2 always
-  const bool single_resident = !switches().no_resident && a->nseg == 1 && a->seg[0].taps == 9 && p.n_blocks == 1 &&
-                               a->seg[0].C % BLOCK_K == 0 &&
+  // 8-row swizzle groups.
+  const bool single_resident = a->nseg == 1 && a->seg[0].taps == 9 && p.n_blocks == 1 && a->seg[0].C % BLOCK_K == 0 &&
                                (long)(a->seg[0].C / BLOCK_K) * 9 * p.block_n * 128 + 2 * A_HALO_BYTES <= SMEM_LIMIT - 2048;
-  const bool pair = pair_mode && (pair_mode == 2 || !single_resident) && p.block_n % 32 == 0 && rbu_num_sms() >= 2 &&
+  const bool pair = !single_resident && p.block_n % 32 == 0 && rbu_num_sms() >= 2 &&
                     (!a->stats || p.n_blocks <= rbu_num_sms() / 2);
   const int b_bytes = (pair ? p.block_n / 2 : p.block_n) * 128;     // one tap's weight tile in ONE CTA's shared memory
   p.tps = p.block_n <= 128 ? 3 : 1;
   p.a_stages = 2;
   // Staged epilogue (TMA stores) when the output is whole 32-column chunks and the staging buffers (8 warps x 4 KB, two per
-  // warp if the weight ring keeps >= 3 stages) fit; RBU_NO_TMA_STORE=1 forces the per-thread stores.
-  const bool can_stage = !switches().no_tma_store && a->Ncols % 32 == 0 && ((uintptr_t)a->y & 15) == 0 && a->y_ld % 8 == 0;
+  // warp if the weight ring keeps >= 3 stages) fit.
+  const bool can_stage = a->Ncols % 32 == 0 && ((uintptr_t)a->y & 15) == 0 && a->y_ld % 8 == 0;
   const int ring_room = SMEM_LIMIT - 2048 - p.a_stages * A_HALO_BYTES;
   p.tma_store = 0;
   p.st_bufs = 0;
@@ -776,9 +760,8 @@ int rbu_conv_halo_launch(const rbu_conv_gemm_args* a, cudaStream_t stream) {
   if (p.b_stages > MAX_B_STAGES) p.b_stages = MAX_B_STAGES;
   {
     // resident weights: one 3x3 segment, one column block, whole operand <= the shared memory left beside 2-3 A stages
-    const int no_res = switches().no_resident;
     const long wbytes = (long)(a->seg[0].C / BLOCK_K) * 9 * b_bytes;
-    if (!no_res && a->nseg == 1 && a->seg[0].taps == 9 && p.n_blocks == 1 && a->seg[0].C % BLOCK_K == 0) {
+    if (a->nseg == 1 && a->seg[0].taps == 9 && p.n_blocks == 1 && a->seg[0].C % BLOCK_K == 0) {
       const int as = 2;   // a third stage does not help (pair 64->64: 759 vs 918 TFLOP/s)
       if (wbytes + as * A_HALO_BYTES <= SMEM_LIMIT - 2048) {
         const long room = SMEM_LIMIT - 2048 - wbytes - as * A_HALO_BYTES;

@@ -23,11 +23,8 @@ int rbu_conv_halo_launch(const rbu_conv_gemm_args* a, cudaStream_t stream);
 int rbu_wgrad_halo_supported(const rbu_wgrad_args* a);
 size_t rbu_wgrad_halo_workspace_bytes(const rbu_wgrad_args* a);
 int rbu_wgrad_halo_launch(const rbu_wgrad_args* a, void* workspace, cudaStream_t stream);
-// wgrad_gemm.cu: the generic kernel restricted to taps [tap_first, tap_end) (tap_end < 0: all), and the split-K reduction
-size_t rbu_wgrad_generic_workspace_bytes(const rbu_wgrad_args* a, int tap_first, int tap_end);
-int rbu_wgrad_generic_launch(const rbu_wgrad_args* a, int tap_first, int tap_end, void* workspace, size_t workspace_bytes,
-                             cudaStream_t stream);
+// wgrad_gemm.cu: the split-K reduction of the weight-gradient partials
 void rbu_wgrad_reduce_launch(const float* partial, int ksplit, int Mtot, int taps, int Ntot, float* out, int accumulate,
-                             cudaStream_t stream, int tap_first = 0, int tap_end = -1);
+                             cudaStream_t stream);
 
 extern "C" size_t rbu_conv_stats_floats(int Ncols);

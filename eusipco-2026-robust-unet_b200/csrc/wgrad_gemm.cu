@@ -16,7 +16,6 @@
 #include "rbu_common.cuh"
 #include "rbu_ptx.cuh"
 #include "tma_host.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -31,7 +30,6 @@ struct WParams {
   int TW, TH, TN;
   int tiles_w, tiles_h, tiles_n, tiles_total;
   int Mtot, Ntot, taps, dil, gather;
-  int tap_first, tap_end;        // taps [tap_first, tap_end) are computed (rbu_wgrad_gemm: all of them)
   int BM, BN, T;                 // block sizes; T taps per work item
   int m_blocks, n_blocks, t_groups, ksplit, items;
   int b_stages, tmem_cols;
@@ -99,8 +97,8 @@ wgrad_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       for (int item = blockIdx.x; item < p.items; item += gridDim.x) {
         int mb, nb, tg, ks;
         decode_item(p, item, mb, nb, tg, ks);
-        const int t_begin = p.tap_first + tg * p.T;
-        const int t_end = min(t_begin + p.T, p.tap_end);
+        const int t_begin = tg * p.T;
+        const int t_end = min(t_begin + p.T, p.taps);
         const int tile0 = (int)((long)ks * p.tiles_total / p.ksplit);
         const int tile1 = (int)((long)(ks + 1) * p.tiles_total / p.ksplit);
         for (int tile = tile0; tile < tile1; ++tile) {
@@ -151,7 +149,7 @@ wgrad_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     for (int item = blockIdx.x; item < p.items; item += gridDim.x, ++it) {
       int mb, nb, tg, ks;
       decode_item(p, item, mb, nb, tg, ks);
-      const int ntap = min(p.tap_first + tg * p.T + p.T, p.tap_end) - (p.tap_first + tg * p.T);
+      const int ntap = min(tg * p.T + p.T, p.taps) - tg * p.T;
       const int tile0 = (int)((long)ks * p.tiles_total / p.ksplit);
       const int tile1 = (int)((long)(ks + 1) * p.tiles_total / p.ksplit);
       ptx::mbar_wait(tempty, (it & 1) ^ 1);
@@ -190,8 +188,8 @@ wgrad_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     for (int item = blockIdx.x; item < p.items; item += gridDim.x, ++it) {
       int mb, nb, tg, ks;
       decode_item(p, item, mb, nb, tg, ks);
-      const int t_begin = p.tap_first + tg * p.T;
-      const int t_end = min(t_begin + p.T, p.tap_end);
+      const int t_begin = tg * p.T;
+      const int t_end = min(t_begin + p.T, p.taps);
       // accumulator row owned by this thread (M=128: lane == row; M=64: rows 16*lg + lane in lanes 0..15)
       int m_local;
       bool row_ok;
@@ -241,7 +239,7 @@ wgrad_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 template <int NCH>
 __global__ void __launch_bounds__(256)
 wgrad_reduce_kernel(const float* __restrict__ partial, int ksplit, int Mtot, int taps, int Ntot,
-                    float* __restrict__ out, int accumulate, int tap_first, int tap_end) {
+                    float* __restrict__ out, int accumulate) {
   constexpr int KL = 256 / NCH;
   constexpr int MAXT = 9;
   __shared__ float lane_sum[KL][MAXT][NCH + 1];
@@ -261,15 +259,15 @@ wgrad_reduce_kernel(const float* __restrict__ partial, int ksplit, int Mtot, int
     for (; k + KL < ksplit; k += 2 * KL) {
 #pragma unroll
       for (int t = 0; t < MAXT; ++t)
-        if (t >= tap_first && t < tap_end) {
+        if (t < taps) {
           acc[t][0] += __ldg(src + (long)k * total + (long)t * Ntot);
           acc[t][1] += __ldg(src + (long)(k + KL) * total + (long)t * Ntot);
         }
     }
-    if (k < ksplit) {
+    if (k < ksplit) {   // 32-bit tap offsets: with 64-bit ones ptxas spills a register pair around this tail
 #pragma unroll
       for (int t = 0; t < MAXT; ++t)
-        if (t >= tap_first && t < tap_end) acc[t][0] += __ldg(src + (long)k * total + (long)t * Ntot);
+        if (t < taps) acc[t][0] += __ldg(src + (long)k * total + t * Ntot);
     }
   }
 #pragma unroll
@@ -285,16 +283,7 @@ wgrad_reduce_kernel(const float* __restrict__ partial, int ksplit, int Mtot, int
   __syncthreads();
   const int nw = min(NCH, Ntot - n0);
   float* o = out + ((long)m * Ntot + n0) * taps;
-  for (int i = threadIdx.x; i < nw * taps; i += 256) {
-    const int t = i % taps;
-    if (t >= tap_first && t < tap_end) o[i] = accumulate ? o[i] + res[i] : res[i];
-  }
-}
-
-bool use_halo(const rbu_wgrad_args* a) {
-  static int no_halo = -1;   // RBU_NO_HALO=1 forces the generic per-tap kernel (A/B comparisons)
-  if (no_halo < 0) no_halo = getenv("RBU_NO_HALO") ? 1 : 0;
-  return !no_halo && rbu_wgrad_halo_supported(a);
+  for (int i = threadIdx.x; i < nw * taps; i += 256) o[i] = accumulate ? o[i] + res[i] : res[i];
 }
 
 int pow2ceil_w(int v) {
@@ -308,11 +297,9 @@ struct Plan {
   size_t ws_bytes;
 };
 
-int make_plan(const rbu_wgrad_args* a, Plan* pl, int tap_first = 0, int tap_end = -1) {
+int make_plan(const rbu_wgrad_args* a, Plan* pl) {
   WParams& p = pl->p;
   memset(&p, 0, sizeof(p));
-  p.tap_first = tap_first;
-  p.tap_end = tap_end < 0 ? a->taps : tap_end;
   p.N = a->N; p.H = a->H; p.W = a->W;
   p.gather = a->gather;
   p.taps = a->taps;
@@ -340,7 +327,7 @@ int make_plan(const rbu_wgrad_args* a, Plan* pl, int tap_first = 0, int tap_end 
   p.T = a->taps == 9 ? 3 : a->taps;   // 3 x 128 or 4 x 128 columns fit the 512-column TMEM
   p.m_blocks = rbu_cdiv(a->Ca, p.BM);
   p.n_blocks = rbu_cdiv(a->Cb, p.BN);
-  p.t_groups = rbu_cdiv(p.tap_end - p.tap_first, p.T);
+  p.t_groups = rbu_cdiv(a->taps, p.T);
   const int base_items = p.m_blocks * p.n_blocks * p.t_groups;
   int ks = rbu_cdiv(2L * rbu_num_sms(), base_items);
   if (ks > p.tiles_total) ks = p.tiles_total;
@@ -369,38 +356,28 @@ int check_args(const rbu_wgrad_args* a) {
 }  // namespace
 
 void rbu_wgrad_reduce_launch(const float* partial, int ksplit, int Mtot, int taps, int Ntot, float* out, int accumulate,
-                             cudaStream_t stream, int tap_first, int tap_end) {
-  if (tap_end < 0) tap_end = taps;
+                             cudaStream_t stream) {
   // 64-column runs (4 split-K lanes) for wide gradients, 32 / 16 columns (8 / 16 lanes) for narrow ones with long chains
   if (Ntot >= 64 && ksplit <= 16)
-    wgrad_reduce_kernel<64><<<Mtot * ((Ntot + 63) / 64), 256, 0, stream>>>(partial, ksplit, Mtot, taps, Ntot, out, accumulate, tap_first, tap_end);
+    wgrad_reduce_kernel<64><<<Mtot * ((Ntot + 63) / 64), 256, 0, stream>>>(partial, ksplit, Mtot, taps, Ntot, out, accumulate);
   else if (Ntot >= 32 && ksplit <= 64)
-    wgrad_reduce_kernel<32><<<Mtot * ((Ntot + 31) / 32), 256, 0, stream>>>(partial, ksplit, Mtot, taps, Ntot, out, accumulate, tap_first, tap_end);
+    wgrad_reduce_kernel<32><<<Mtot * ((Ntot + 31) / 32), 256, 0, stream>>>(partial, ksplit, Mtot, taps, Ntot, out, accumulate);
   else
-    wgrad_reduce_kernel<16><<<Mtot * ((Ntot + 15) / 16), 256, 0, stream>>>(partial, ksplit, Mtot, taps, Ntot, out, accumulate, tap_first, tap_end);
+    wgrad_reduce_kernel<16><<<Mtot * ((Ntot + 15) / 16), 256, 0, stream>>>(partial, ksplit, Mtot, taps, Ntot, out, accumulate);
 }
 
 extern "C" size_t rbu_wgrad_workspace_bytes(const rbu_wgrad_args* a) {
   if (check_args(a) != RBU_OK) return 0;
-  if (use_halo(a)) return rbu_wgrad_halo_workspace_bytes(a);
+  if (rbu_wgrad_halo_supported(a)) return rbu_wgrad_halo_workspace_bytes(a);
   Plan pl;
   make_plan(a, &pl);
   return pl.ws_bytes;
 }
 
-// The generic kernel restricted to taps [tap_first, tap_end) (tap_end < 0: all).  Its only caller, rbu_wgrad_gemm, passes
-// the whole tap range; the halo kernels (wgrad_halo.cu) compute all nine taps themselves and never call this.
-size_t rbu_wgrad_generic_workspace_bytes(const rbu_wgrad_args* a, int tap_first, int tap_end) {
-  Plan pl;
-  make_plan(a, &pl, tap_first, tap_end);
-  return pl.ws_bytes;
-}
-
-int rbu_wgrad_generic_launch(const rbu_wgrad_args* a, int tap_first, int tap_end, void* workspace, size_t workspace_bytes,
-                             cudaStream_t stream) {
+static int rbu_wgrad_generic_launch(const rbu_wgrad_args* a, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   int rc;
   Plan pl;
-  make_plan(a, &pl, tap_first, tap_end);
+  make_plan(a, &pl);
   WParams& p = pl.p;
   RBU_CHECK_ARG(workspace && workspace_bytes >= pl.ws_bytes && ((uintptr_t)workspace & 15) == 0,
                 "rbu_wgrad_gemm: workspace too small (%zu < %zu)", workspace_bytes, pl.ws_bytes);
@@ -449,7 +426,7 @@ int rbu_wgrad_generic_launch(const rbu_wgrad_args* a, int tap_first, int tap_end
   const int grid = p.items < rbu_num_sms() ? p.items : rbu_num_sms();
   wgrad_gemm_kernel<<<grid, NUM_THREADS, smem_bytes, stream>>>(tmA, tmB, p);
   RBU_CHECK_LAUNCH();
-  rbu_wgrad_reduce_launch(p.partial, p.ksplit, p.Mtot, p.taps, p.Ntot, a->out, a->accumulate, stream, p.tap_first, p.tap_end);
+  rbu_wgrad_reduce_launch(p.partial, p.ksplit, p.Mtot, p.taps, p.Ntot, a->out, a->accumulate, stream);
   RBU_CHECK_LAUNCH();
   return RBU_OK;
 }
@@ -460,10 +437,10 @@ extern "C" int rbu_wgrad_gemm(const rbu_wgrad_args* a, void* workspace, size_t w
   if (rc) return rc;
   RBU_CHECK_ARG(a->a && a->b && a->out && ((uintptr_t)a->a & 15) == 0 && ((uintptr_t)a->b & 15) == 0,
                 "rbu_wgrad_gemm: null or misaligned pointer");
-  if (use_halo(a)) {
+  if (rbu_wgrad_halo_supported(a)) {
     RBU_CHECK_ARG(workspace && workspace_bytes >= rbu_wgrad_halo_workspace_bytes(a) && ((uintptr_t)workspace & 15) == 0,
                   "rbu_wgrad_gemm: workspace too small");
     return rbu_wgrad_halo_launch(a, workspace, stream);
   }
-  return rbu_wgrad_generic_launch(a, 0, -1, workspace, workspace_bytes, stream);
+  return rbu_wgrad_generic_launch(a, workspace, workspace_bytes, stream);
 }

@@ -531,15 +531,11 @@ void plan(const rbu_wgrad_args* a, HWParams* p) {
   p->Cin = a->Cb;
   {
     // Block shape: 128 output x 32 input channels (second form, balanced shared-memory operand fetch) whenever the channel
-    // counts allow it, else 64 x 64 (the 64-output-channel level).  RBU_WGRAD_V1=1 forces the first form (A/B measurements).
-    static int v1 = -1;
-    if (v1 < 0) v1 = getenv("RBU_WGRAD_V1") ? 1 : 0;
-    const bool form2 = !v1 && a->Ca % 128 == 0 && a->Cb % 32 == 0;
+    // counts allow it, else 64 x 64 (the 64-output-channel level).
+    const bool form2 = a->Ca % 128 == 0 && a->Cb % 32 == 0;
     p->OB = form2 ? 128 : 64;
     p->CB = form2 ? 32 : 64;
-    static int pair = -1;
-    if (pair < 0) pair = getenv("RBU_WGRAD_NOPAIR") ? 0 : 1;     // RBU_WGRAD_NOPAIR=1: second form everywhere (A/B measurements)
-    if (form2 && pair && a->Ca % 256 == 0) p->OB = 256;          // third form: a CTA pair per item
+    if (form2 && a->Ca % 256 == 0) p->OB = 256;          // third form: a CTA pair per item
   }
   p->cin_blocks = rbu_cdiv(a->Cb, p->CB);
   p->cout_blocks = rbu_cdiv(a->Ca, p->OB);

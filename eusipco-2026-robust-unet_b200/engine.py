@@ -8,7 +8,6 @@ Layout: activations are NHWC bf16 (`View`s, possibly channel slices of a wider b
 from __future__ import annotations
 
 import ctypes
-import os
 from collections import namedtuple
 from ctypes import c_void_p
 
@@ -62,25 +61,9 @@ class Engine:
         self.grad_alloc = None        # optional callable(name, shape) -> fp32 tensor to receive that parameter's gradient
                                       # (parallel.DataParallel: a slice of a flat all-reduce bucket), or None
         self._saving = False
-        # Weight gradients on a side stream (see wgrad()).  RBU_NO_OVERLAP=1 keeps them on the compute stream: used by the
-        # profiling tools, which need per-kernel times that are not inflated by a co-running kernel.
-        self.overlap_wgrad = os.environ.get("RBU_NO_OVERLAP") is None
-        # BatchNorm batch statistics of the 1x1 (shortcut, attention-gate, stem, dilated-block) convolutions from the generic
-        # kernel's staged epilogue (rbu_conv_gemm stats=...) instead of a separate pass over the stored tensor.  Round 1's
-        # warp-transpose reduction cost as much as the pass it saved (44.9 vs 45.0 ms/step); since the statistics are read
-        # off the staged outputs (lane = channel pair, register accumulators for the life of the CTA) they are on.
-        # RBU_NO_FUSE_BN=1 restores the separate passes (A/B runs).
-        self.fuse_bn_stats = os.environ.get("RBU_NO_FUSE_BN") is None
-        # Per-image statistics (sum, sum of squares, max, min per half-tile) from the 3x3 halo kernel's epilogue: BatchNorm
-        # batch statistics and ChannelAttention's pooled inputs without re-reading the conv output.  Measured on B200: in
-        # the training step (batch 64, 256^2) the 18 statistics passes it replaces cost 1.34 ms, the longer epilogues 0.4 ms
-        # and the reduction of the partials 0.35 ms.  Since the statistics are read off the staged outputs (round 2: half the
-        # epilogue cost) they are used from 64 output channels up -- 64->64 at 256^2: +0.059 ms in the convolution against a
-        # 0.115-0.151 ms statistics pass, step -0.2 to -0.4 ms (tools/tile_stats_ab.py) -- and in training mode only
-        # (inference at 1024^2, round 2: statistics pass -1.9 ms, convolutions +1.7 ms -- no gain).
-        self.fuse_tile_stats = True
-        self.tile_stats_eval = False
-        self.tile_stats_min_c = 64
+        # Weight gradients on a side stream (see wgrad()).  The profiling tools turn this off: they need per-kernel times
+        # that are not inflated by a co-running kernel.
+        self.overlap_wgrad = True
         self._ws = None
         self._defer_counters = False     # whole-model forward: the 39 num_batches_tracked increments become one launch
         self._pending_counters = []
@@ -211,9 +194,17 @@ class Engine:
             self._bump(bn)
         return out
 
-    def tile_stats_ok(self, H, W, C):
-        """The 3x3 halo kernel can emit the per-image statistics of its output (see bn_stats_tiles)."""
-        return self.fuse_tile_stats and H >= 16 and W >= 16 and C % 32 == 0 and self.tile_stats_min_c <= C <= 2048
+    @staticmethod
+    def tile_stats_ok(H, W, C):
+        """Whether a training forward takes this 3x3 convolution's per-image statistics (sum, sum of squares, max, min per
+        half-tile) from the halo kernel's epilogue (see bn_stats_tiles): BatchNorm batch statistics and ChannelAttention's
+        pooled inputs without re-reading the conv output.  Measured on B200: in the training step (batch 64, 256^2) the 18
+        statistics passes it replaces cost 1.34 ms, the longer epilogues 0.4 ms and the reduction of the partials 0.35 ms.
+        Since the statistics are read off the staged outputs (round 2: half the epilogue cost) they are used from 64 output
+        channels up -- 64->64 at 256^2: +0.059 ms in the convolution against a 0.115-0.151 ms statistics pass, step -0.2 to
+        -0.4 ms (profiles/r02_tile_stats_smem.log) -- and in training mode only (inference at 1024^2, round 2: statistics
+        pass -1.9 ms, convolutions +1.7 ms -- no gain)."""
+        return H >= 16 and W >= 16 and C % 32 == 0 and 64 <= C <= 2048
 
     def tile_stats_buf(self, N, H, W, C, device):
         return torch.empty(_lib.lib().rbu_conv_tile_stats_floats(N, H, W, C), dtype=torch.float32, device=device)
@@ -256,7 +247,11 @@ class Engine:
         return out
 
     def conv_stats_buf(self, Ncols, device):
-        """Scratch for the BatchNorm partial sums a convolution's epilogue emits (training only)."""
+        """Scratch for the BatchNorm partial sums a convolution's epilogue emits (training only).  Training takes the batch
+        statistics of the 1x1 (shortcut, attention-gate, stem, dilated-block) convolutions from the generic kernel's staged
+        epilogue instead of a separate pass over the stored tensor.  Round 1's warp-transpose reduction cost as much as the
+        pass it saved (44.9 vs 45.0 ms/step); read off the staged outputs (lane = channel pair, register accumulators for
+        the life of the CTA) they win (profiles/r02_bn_fuse_ab.log)."""
         return torch.empty(_lib.lib().rbu_conv_stats_floats(Ncols), dtype=torch.float32, device=device)
 
     def bn_from_conv(self, part, Ncols, col_off, C, count, bn: nn.BatchNorm2d, off=0, out=None):
@@ -365,14 +360,13 @@ class Engine:
         proj = not isinstance(blk.shortcut, nn.Identity)
         s = {"name": name, "x": x, "N": N, "H": H, "W": W, "C": C, "proj": proj, "patches": stem_patches}
         bns = bn1 = None
-        fuse = training and self.fuse_bn_stats
         if stem_patches is not None:
             y12 = self.new(N, H, W, 2 * C, dev)
-            st12 = self.conv_stats_buf(2 * C, dev) if fuse else None
+            st12 = self.conv_stats_buf(2 * C, dev) if training else None
             conv_gemm(N, H, W, [(stem_patches, self._packs[(id(blk.conv1.weight), 4)], 1, 0, False)], 2 * C, y12,
                       flops=2.0 * N * H * W * C * 10 * blk.conv1.in_channels, stats=st12)
             y1, ys = y12.slice(0, C), y12.slice(C, C)
-            if fuse:
+            if training:
                 bn1 = self.bn_from_conv(st12, 2 * C, 0, C, P, blk.bn1)
                 bns = self.bn_from_conv(st12, 2 * C, C, C, P, blk.shortcut[1])
                 self._bump(blk.bn1)
@@ -381,28 +375,24 @@ class Engine:
             folded = not training and not self._saving   # inference: BN1 + ReLU ride in conv1's epilogue, no y1
             y1 = None if folded else self.new(N, H, W, C, dev)
             # bn1 needs the batch statistics only (no per-image pooling): per-CTA register accumulators in the convolution's
-            # epilogue (no per-tile exchange, no second stage over tiles); per-tile statistics when those are switched off
-            use_ts1 = training and not folded and not fuse and self.tile_stats_ok(H, W, C)
-            st1 = self.conv_stats_buf(C, dev) if fuse else None
+            # epilogue (no per-tile exchange, no second stage over tiles)
+            st1 = self.conv_stats_buf(C, dev) if training else None
             if folded:
                 bn1 = self.bn_eval_affine(blk.bn1, x)
                 a1 = self.new(N, H, W, C, dev)
                 conv_gemm(N, H, W, [(x, self.pack(blk.conv1.weight, 0), 9, 1, False)], C, a1, scale=bn1["scale"],
                           bias=bn1["shift"], relu=C)
             else:
-                ts1 = self.tile_stats_buf(N, H, W, C, dev) if use_ts1 else None
-                conv_gemm(N, H, W, [(x, self.pack(blk.conv1.weight, 0), 9, 1, False)], C, y1, stats=st1, tile_stats=ts1)
-                if ts1 is not None:
-                    bn1 = self.bn_stats_tiles(ts1, N, H, W, C, blk.bn1, training)
+                conv_gemm(N, H, W, [(x, self.pack(blk.conv1.weight, 0), 9, 1, False)], C, y1, stats=st1)
             if st1 is not None:
                 bn1 = self.bn_from_conv(st1, C, 0, C, P, blk.bn1)
                 self._bump(blk.bn1)
             ys = None
             if proj:
                 ys = self.new(N, H, W, C, dev)
-                sts = self.conv_stats_buf(C, dev) if fuse else None
+                sts = self.conv_stats_buf(C, dev) if training else None
                 conv_gemm(N, H, W, [(x, self.pack(blk.shortcut[0].weight, 0), 1, 0, False)], C, ys, stats=sts)
-                if fuse:
+                if training:
                     bns = self.bn_from_conv(sts, C, 0, C, P, blk.shortcut[1])
                     self._bump(blk.shortcut[1])
         if y1 is not None and bn1 is None:
@@ -413,7 +403,7 @@ class Engine:
             call("rbu_affine_act", _vp(y1), y1.ld, _vp(a1), a1.ld, P, HW, C, _p(bn1["scale"]), _p(bn1["shift"]), _p(drop), 1,
                  stream_ptr())
         y2 = self.new(N, H, W, C, dev)
-        ts2 = self.tile_stats_buf(N, H, W, C, dev) if ((training or self.tile_stats_eval) and self.tile_stats_ok(H, W, C)) else None
+        ts2 = self.tile_stats_buf(N, H, W, C, dev) if training and self.tile_stats_ok(H, W, C) else None
         conv_gemm(N, H, W, [(a1, self.pack(blk.conv2.weight, 0), 9, 1, False)], C, y2, tile_stats=ts2)
         if ts2 is not None:
             bn2 = self.bn_stats_tiles(ts2, N, H, W, C, blk.bn2, training, pool=True)
@@ -541,12 +531,11 @@ class Engine:
         C, F = skip.C, gate.W_g[0].out_channels
         HW, P = H * W, N * H * W
         yg, yx = self.new(N, H, W, F, dev), self.new(N, H, W, F, dev)
-        fuse = training and self.fuse_bn_stats
-        stg = self.conv_stats_buf(F, dev) if fuse else None
-        stx = self.conv_stats_buf(F, dev) if fuse else None
+        stg = self.conv_stats_buf(F, dev) if training else None
+        stx = self.conv_stats_buf(F, dev) if training else None
         conv_gemm(N, H, W, [(g, self.pack(gate.W_g[0].weight, 0), 1, 0, False)], F, yg, bias=gate.W_g[0].bias, stats=stg)
         conv_gemm(N, H, W, [(skip, self.pack(gate.W_x[0].weight, 0), 1, 0, False)], F, yx, bias=gate.W_x[0].bias, stats=stx)
-        if fuse:
+        if training:
             bg = self.bn_from_conv(stg, F, 0, F, P, gate.W_g[1])
             bx = self.bn_from_conv(stx, F, 0, F, P, gate.W_x[1])
             self._bump(gate.W_g[1])
@@ -611,15 +600,14 @@ class Engine:
         ycat = self.new(N, H, W, C, dev)
         convs = (blk.conv1, blk.conv2, blk.conv3, blk.conv4)
         bn = None
-        fuse = training and self.fuse_bn_stats
         for i, cv in enumerate(convs):
             taps = 1 if i == 0 else 9
-            sti = self.conv_stats_buf(Cq, dev) if fuse else None
+            sti = self.conv_stats_buf(Cq, dev) if training else None
             conv_gemm(N, H, W, [(x, self.pack(cv.weight, 0), taps, cv.dilation[0], False)], Cq, ycat.slice(i * Cq, Cq),
                       bias=cv.bias, stats=sti)
-            if fuse:
+            if training:
                 bn = self.bn_from_conv(sti, Cq, 0, Cq, P, blk.bn, off=i * Cq, out=bn)
-        if fuse:
+        if training:
             self._bump(blk.bn)
         else:
             bn = self.bn_stats(ycat, N, HW, blk.bn, training)

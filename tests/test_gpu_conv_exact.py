@@ -97,14 +97,14 @@ def _row(id, op, N, H, W, cin, cout, kernels, k=3, dil=1, **epi):
 
 # Forward and data-gradient rows.  op: fwd (pack mode 0), dgrad (mode 1), dgrad2 (3x3 dgrad + 1x1 shortcut dgrad in one
 # accumulator), convT (ConvTranspose2d forward, scatter into the second half of a concat buffer), convT_dgrad (gather).
-# Halo selection: conv_halo.cu:705-720 (rbu_conv_halo_supported: 3x3 dil 1 / 1x1 segments, H, W >= 16, no scatter /
-# gather); block_n conv_halo.cu:734-735; single-CTA resident vs pair conv_halo.cu:754-758 (single CTA only when the whole
+# Halo selection: conv_halo.cu:692-707 (rbu_conv_halo_supported: 3x3 dil 1 / 1x1 segments, H, W >= 16, no scatter /
+# gather); block_n conv_halo.cu:721-722; single-CTA resident vs pair conv_halo.cu:739-742 (single CTA only when the whole
 # operand is resident: one 3x3 segment, one column block, C % 64 == 0, C/64 * block_n <= 96); staging buffers
-# conv_halo.cu:764-775 (streamed) and :777-792 (resident: 2 / 1 / 0 buffers by the room left).
-# Generic: conv_gemm.cu:617-622 (everything the halo kernel refuses), :628-642 (tiles), :644 (block_n), :665-673 (TMA
-# stores), :679-686 (resident weights).
+# conv_halo.cu:748-760 (streamed) and :761-776 (resident: 2 / 1 / 0 buffers by the room left).
+# Generic: conv_gemm.cu:616-617 (everything the halo kernel refuses), :623-637 (tiles), :639 (block_n), :660-666 (TMA
+# stores), :672-675 (resident weights).
 CONV_ROWS = [
-    # --- single-CTA halo kernel, resident weights (conv_halo.cu:754-756, :781-791)
+    # --- single-CTA halo kernel, resident weights (conv_halo.cu:739-740, :764-774)
     _row("halo1_64to64_res_1buf", "fwd", 2, 32, 32, 64, 64, [HALO], bias=True),          # 72 KB weights: 1 buffer
     _row("halo1_64to32_res_2buf", "fwd", 3, 16, 16, 64, 32, [HALO], bias=True),          # 36 KB weights: 2 buffers
     _row("halo1_64to96_res_direct", "fwd", 2, 32, 16, 64, 96, [HALO], bias=True),       # 96: no room, per-thread
@@ -117,13 +117,15 @@ CONV_ROWS = [
     _row("pair_1024to1024_one_tile", "fwd", 2, 16, 16, 1024, 1024, [PAIR]),              # one tile: block_n 256
     _row("pair_256to1024_one_tile_odd", "fwd", 3, 16, 16, 256, 1024, [PAIR], bias=True), # 3 tiles: idle CTA, 256 columns
     _row("pair_dgrad_128to64", "dgrad", 2, 32, 32, 64, 128, [PAIR]),                     # pack mode 1, 2 slabs -> 64 columns
-    # --- per-thread stores (Ncols % 32 != 0: conv_halo.cu:764)
+    # --- per-thread stores (Ncols % 32 != 0: conv_halo.cu:748)
     _row("halo1_n40_ragged", "fwd", 2, 24, 20, 64, 40, [HALO], bias=True),               # block_n 64, resident
     _row("halo1_n72", "fwd", 2, 16, 16, 64, 72, [HALO], addend=True),                    # block_n 96: resident
     _row("pair_n40", "fwd", 2, 16, 32, 128, 40, [PAIR], bias=True),                      # 2 slabs: pair, resident
     _row("pair_n72_streamed", "fwd", 1, 32, 32, 256, 72, [PAIR], addend=True),           # 4 slabs x 96: streamed
+    _row("pair_dgrad_n40_direct", "dgrad", 2, 32, 32, 40, 128, [PAIR]),                  # 2 slabs x 64: pair
     # --- two segments (conv1 3x3 dgrad + shortcut 1x1 dgrad): not resident -> pair, block_n 64, 2 staging buffers
     _row("pair_two_segments_ragged", "dgrad2", 2, 20, 36, 64, 128, [PAIR]),
+    _row("pair_two_segments_n40_direct", "dgrad2", 2, 20, 36, 40, 128, [PAIR]),          # Ncols 40: per-thread stores
     # --- halo epilogue: single CTA (64 -> 64 resident) and pair (128 -> 128 streamed)
     _row("epi_bias_single", "fwd", 2, 32, 32, 64, 64, [HALO], bias=True),
     _row("epi_bias_pair", "fwd", 2, 32, 32, 128, 128, [PAIR], bias=True),
@@ -141,6 +143,7 @@ CONV_ROWS = [
     _row("stats_single_direct", "fwd", 2, 32, 16, 64, 96, [HALO], stats=True, sparse=True),
     _row("stats_pair_one_block", "fwd", 2, 32, 32, 128, 128, [PAIR], stats=True, sparse=True),
     _row("stats_pair_four_blocks", "fwd", 2, 32, 32, 128, 512, [PAIR], stats=True, sparse=True),
+    _row("stats_pair_direct_n72", "fwd", 2, 32, 32, 128, 72, [PAIR], stats=True, sparse=True),   # <= 128 columns
     # --- halo epilogue, per-image tile statistics on ragged 40 x 24 images
     _row("tile_stats_single_staged", "fwd", 2, 40, 24, 64, 64, [HALO], tile_stats=True, sparse=True),
     _row("tile_stats_single_direct", "fwd", 2, 40, 24, 64, 96, [HALO], tile_stats=True, sparse=True),
@@ -151,6 +154,7 @@ CONV_ROWS = [
     _row("gen_3x3_dil2_streamed", "fwd", 2, 16, 16, 64, 64, [GEN], dil=2, bias=True),    # 9 k-blocks x 64: 72 KB streamed
     _row("gen_3x3_dil4_resident", "fwd", 2, 32, 32, 32, 32, [GEN], dil=4),               # 9 x 32 columns: 36 KB resident
     _row("gen_dgrad_dil2", "dgrad", 2, 16, 16, 64, 128, [GEN], dil=2),
+    _row("gen_dgrad_dil2_n40_direct", "dgrad", 2, 16, 16, 40, 128, [GEN], dil=2),       # per-thread stores
     _row("gen_3x3_8x8_tn2", "fwd", 3, 8, 8, 128, 64, [GEN], bias=True),                  # TW = TH = 8, TN = 2, N odd
     _row("gen_3x3_4x4_tn8", "fwd", 5, 4, 4, 64, 64, [GEN], addend=True),                 # TN = 8 images per tile
     _row("gen_3x3_1x1_130_images", "fwd", 130, 1, 1, 64, 64, [GEN]),                     # TN = 128: two tiles
@@ -160,7 +164,8 @@ CONV_ROWS = [
     _row("gen_scale_relu_prefix", "fwd", 2, 16, 16, 128, 64, [GEN], k=1, scale=True, bias=True, relu=16),
     _row("gen_stats_staged", "fwd", 3, 24, 40, 64, 128, [GEN], k=1, stats=True, sparse=True),
     _row("gen_stats_direct_n40", "fwd", 3, 24, 40, 64, 40, [GEN], k=1, stats=True, sparse=True),
-    # --- ConvTranspose2d(2, s=2) (conv_gemm.cu:670-671: TMA stores need Cout % 64 == 0)
+    _row("gen_stats_direct_two_blocks", "fwd", 2, 16, 16, 64, 264, [GEN], k=1, stats=True, sparse=True),  # 256 + 8
+    # --- ConvTranspose2d(2, s=2) (conv_gemm.cu:663-664: TMA stores need Cout % 64 == 0)
     _row("convT_scatter_c64_tma", "convT", 2, 8, 8, 128, 64, [GEN], bias=True),
     _row("convT_scatter_c32_direct", "convT", 2, 8, 8, 64, 32, [GEN], bias=True),
     _row("convT_dgrad_gather", "convT_dgrad", 2, 8, 8, 128, 64, [GEN]),
@@ -292,10 +297,10 @@ def test_gpu_reference_matches_cpu_reference():
         assert torch.equal(cpu, gpu), name
 
 
-# Weight-gradient rows.  Halo kernels: wgrad_halo.cu:572-574 (3x3 dil 1, H >= 8, W >= 16), forms wgrad_halo.cu:533-543
+# Weight-gradient rows.  Halo kernels: wgrad_halo.cu:568-570 (3x3 dil 1, H >= 8, W >= 16), forms wgrad_halo.cu:532-539
 # (form 2 when Cout % 128 == 0 and Cin % 32 == 0, the pair form when also Cout % 256 == 0, else form 1); split-K from the
-# cost model wgrad_halo.cu:547-566.  Generic kernel: wgrad_gemm.cu:294-298 and :311-357 (ksplit = ceil(2 * SMs /
-# items), capped by the pixel tiles).  Reduction kernel: wgrad_gemm.cu:371-381 (<64> for Cin >= 64 and ksplit <= 16, <32>
+# cost model wgrad_halo.cu:543-563.  Generic kernel: wgrad_gemm.cu:440-445 and :300-344 (ksplit = ceil(2 * SMs /
+# items), capped by the pixel tiles).  Reduction kernel: wgrad_gemm.cu:358-367 (<64> for Cin >= 64 and ksplit <= 16, <32>
 # for Cin >= 32 and ksplit <= 64, else <16>).  The ksplit values in the comments are for 148 SMs.
 WGRAD_ROWS = [
     _row("w_form1_64x64", "wgrad", 2, 32, 32, 64, 64, [W1, R64]),                      # ksplit 2

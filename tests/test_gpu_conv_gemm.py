@@ -180,28 +180,6 @@ def test_invalid_arguments_raise():
         ops.conv_gemm(1, 4, 4, [(ops.View(x), w, 1, 1, False)], 60, ops.View(y))   # Ncols % 8
 
 
-@pytest.mark.parametrize("switch", ["RBU_CONV_PAIR", "RBU_CONV_NOPAIR", "RBU_NO_TMA_STORE"])
-def test_halo_kernel_forced_variants(switch):
-    """The library picks the single-CTA or the CTA-pair 3x3 kernel by shape and stages its outputs for TMA stores when
-    the buffers fit; the switches are read once per process, so the 3x3 cases, the data-gradient and the two-segment case
-    are repeated in a child process with each variant forced (pair everywhere / never / per-thread stores)."""
-    import os
-    import subprocess
-    import sys
-    if os.environ.get("RBU_CONV_CHILD"):
-        pytest.skip("child run")
-    env = dict(os.environ, RBU_CONV_CHILD="1")
-    env.pop("RBU_CONV_PAIR", None)
-    env.pop("RBU_CONV_NOPAIR", None)
-    env[switch] = "1"
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-m", "gpu", "-x",
-                        "-k", "3x3 or dgrad or two_segment or statistics", "-p", "no:cacheprovider"],
-                       env=env, capture_output=True, text=True, timeout=600,
-                       cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout
-
-
 @pytest.mark.parametrize("shape", [
     # N, H, W, Cin, Ncols, bias
     (3, 32, 32, 64, 64, False),      # shortcut-like
