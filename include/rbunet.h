@@ -404,6 +404,41 @@ typedef struct { int scene, op, y0, x0, focus, pad; long long r; } rbu_patch_job
 int rbu_sample_patches(const rbu_patch_src* srcs_device, int S, const rbu_patch_job* jobs_device, int B, int ph, int pw,
                        int n_channels, float* images_out, uint8_t* masks_out, int* jobs_out, void* stream);
 
+/* ------------------------------------------------------------------ distance transform and coastline distances
+ * How far the predicted coastline is from the true one, which the area metrics above (IoU, F1) do not measure.  No
+ * reference counterpart: the reference stops at the coastline band (predict_coastline.py:595-602).
+ *
+ * rbu_edt: the exact squared Euclidean distance transform of B feature images features_u8 [B][H][W] (nonzero = feature),
+ * 1 <= H, W <= 32768, B <= 65535:  dist2_out int32 [B][H][W],  D(y,x) = min over feature pixels (v,u) of
+ * (y-v)^2 + (x-u)^2;  0 on the features, -1 everywhere in an image without a feature pixel.  Equal to
+ * rint(scipy.ndimage.distance_transform_edt(F == 0) ** 2).  Separable (Meijster et al. 2000) with integer intersections:
+ * four launches whatever the distances.  workspace: rbu_edt_workspace_bytes(B, H, W) bytes, 16-byte aligned (about
+ * 8.3 bytes per pixel). */
+size_t rbu_edt_workspace_bytes(int B, int H, int W);
+int rbu_edt(const uint8_t* features_u8, int B, int H, int W, int32_t* dist2_out, void* workspace, size_t workspace_bytes,
+            void* stream);
+/* rbu_coastline_stats: per image b of pred / target [B][H][W] (B <= 32767, 1 <= H, W <= 32768):
+ *  - water: kind RBU_KIND_F32 (float32): pred p > threshold (strict), target t != 0 (the rules of rbu_confusion_counts);
+ *    kind RBU_KIND_U8 (uint8, also bool): nonzero.
+ *  - coastline of a water mask: the non-water pixels with a water pixel among their four in-image neighbours, i.e.
+ *    rbu_coastline_mask(water, ksize 3) != 0.  P = coastline of pred, G = coastline of target.
+ *  - direction 0 (pred -> target): samples d2 = D_G at the pixels of P; direction 1 (target -> pred): D_P at those of G.
+ *  stats_out float64 [B][2][5 + T], per (image, direction):
+ *    [0] n, the number of samples (pixels of the source coastline);
+ *    [1] the sum of sqrt((double)d2), fixed order (bit-identical run to run, and for an image alone or in a batch);
+ *    [2] max d2;  [3], [4] the order statistics of d2 at ranks floor((n-1)*0.95) and the next one (both n-1 at the
+ *        end), between which numpy's "linear" 95th percentile interpolates;
+ *    [5 + k] the count of samples with d2 <= tol_d2[k].
+ *  Without a distance (n = 0, or the opposite coastline is empty) [1]-[4] are -1 and the counts 0.  tol_d2 is a
+ *  HOST array of T (0..8) non-negative thresholds.  Workspace: rbu_coastline_stats_workspace_bytes(B, H, W) bytes,
+ *  16-byte aligned.  Nine launches and one memset whatever B, H and W. */
+#define RBU_KIND_F32 (0)
+#define RBU_KIND_U8 (1)
+size_t rbu_coastline_stats_workspace_bytes(int B, int H, int W);
+int rbu_coastline_stats(const void* pred, int pred_kind, const void* target, int target_kind, float threshold, int B, int H,
+                        int W, const int* tol_d2, int T, double* stats_out, void* workspace, size_t workspace_bytes,
+                        void* stream);
+
 #ifdef __cplusplus
 }
 #endif
