@@ -439,6 +439,42 @@ int rbu_coastline_stats(const void* pred, int pred_kind, const void* target, int
                         int W, const int* tol_d2, int T, double* stats_out, void* workspace, size_t workspace_bytes,
                         void* stream);
 
+/* ------------------------------------------------------------------ connected components of water masks
+ * Cleaning a predicted mask before its coastline is measured or traced: every false blob adds its own ring of coastline
+ * (cv2.findContours at predict_coastline.py:605-616 turns each into a polygon).  Block-based union-find (Playne & Hawick
+ * 2018; Allegretti et al. 2019) whose root is the minimum per-image linear index: every output is a function of the mask
+ * alone, the same bits run to run and for an image alone or inside a batch.  Integer atomics only; 64-bit image offsets.
+ *  - mask: [B][H][W], 1 <= B <= 65535, 1 <= H, W <= 32768; water is kind RBU_KIND_F32: p > threshold (strict), kind
+ *    RBU_KIND_U8 (uint8, also bool): nonzero (the pred rule of rbu_coastline_stats).
+ *  - connectivity 4 (edge neighbours) or 8 (edge and corner neighbours).
+ *
+ * rbu_label_components: labels_out int32 [B][H][W], 0 on land, components numbered 1..n_b in raster order of their first
+ * pixel (minimum y*W + x) = scipy.ndimage.label(water, generate_binary_structure(2, connectivity == 4 ? 1 : 2));
+ * counts_out int32 [B] = n_b.  Workspace: rbu_label_workspace_bytes(B, H, W) bytes (about 4.1 per pixel), 16-byte
+ * aligned.  Six launches whatever the content: tile union-find, tile-border unions, flatten + root counts, per-image
+ * scan, raster ranks, label write. */
+size_t rbu_label_workspace_bytes(int B, int H, int W);
+int rbu_label_components(const void* mask, int kind, float threshold, int B, int H, int W, int connectivity,
+                         int32_t* labels_out, int32_t* counts_out, void* workspace, size_t workspace_bytes, void* stream);
+/* rbu_component_stats: per component of labels [B][H][W] (as rbu_label_components writes them), into row
+ * row_offsets[b] + label - 1 of stats_out int64 [rows][7]: left, top, right, bottom (inclusive), area, sum of x, sum of y.
+ * row_offsets: DEVICE int64 [B + 1]; rows row_offsets[0] .. row_offsets[B] - 1 are written, no others.  Labels outside
+ * [1, row_offsets[b + 1] - row_offsets[b]] are ignored.  Width = right - left + 1 and height = bottom - top + 1 give
+ * OpenCV's CC_STAT layout; the centroid is (sum x / area, sum y / area).  Two launches whatever the content; one set of
+ * atomics per (32 x 32 tile, component). */
+int rbu_component_stats(const int32_t* labels, int B, int H, int W, const int64_t* row_offsets, int64_t* stats_out,
+                        void* stream);
+/* rbu_remove_small_regions: out_u8 [B][H][W] 0/1.  Step 1: every water component (at `connectivity`) with fewer than
+ * min_water pixels becomes land.  Step 2, on the result of step 1: every land component with fewer than min_land pixels
+ * becomes water.  Regions touching the image border get no special treatment; a threshold of 0 or 1 makes its step the
+ * identity.  Workspace: rbu_remove_small_regions_workspace_bytes(B, H, W) bytes (about 8 per pixel), 16-byte aligned.
+ * Eight launches whatever the content: per step tile union-find with tile areas, tile-border unions, flatten + area
+ * aggregation at the roots, write. */
+size_t rbu_remove_small_regions_workspace_bytes(int B, int H, int W);
+int rbu_remove_small_regions(const void* mask, int kind, float threshold, int B, int H, int W, int connectivity,
+                             int min_water, int min_land, uint8_t* out_u8, void* workspace, size_t workspace_bytes,
+                             void* stream);
+
 #ifdef __cplusplus
 }
 #endif
