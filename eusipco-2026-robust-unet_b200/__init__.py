@@ -11,11 +11,13 @@ Drop-in surface (reference: /root/reference/Main_Final.py):
   distance_transform(features)                              exact squared Euclidean distance transform
   remove_small_regions(mask, min_water, min_land)           drop small water blobs, fill small land specks
   label_components(mask, connectivity) / component_stats    connected components (scipy / OpenCV numbering and stats)
+  find_contours(mask, approx)                               outer contours, bit for bit with cv2.findContours(RETR_EXTERNAL)
 Everything below that surface is hand-written CUDA in csrc/ reached through the C ABI of
 librbunet.so (include/rbunet.h).  There is no CPU fallback.
 """
 from . import _lib  # noqa: F401
 from .components import component_stats, label_components, remove_small_regions  # noqa: F401
+from .contours import find_contours  # noqa: F401
 from .distance import coastline_metrics, coastline_stats, distance_transform  # noqa: F401
 from .loss import (METRIC_KEYS, RobustBCEDiceLoss, batch_metrics, calculate_metrics,  # noqa: F401
                    class_confusion_counts, class_metrics, confusion_counts, metrics_from_counts)
@@ -28,4 +30,4 @@ from .tiled import predict_tiled  # noqa: F401
 from .unet import CrossEntropyArgmaxLoss, UNet  # noqa: F401
 
 __all__ = ["RobustUNet", "ResidualBlock", "AttentionGate", "DilatedBlock", "RobustBCEDiceLoss", "calculate_metrics", "batch_metrics", "confusion_counts", "class_confusion_counts", "class_metrics",
-           "metrics_from_counts", "METRIC_KEYS", "View", "preprocess", "resize", "enhance_image", "coastline_mask", "predict_tiled", "PatchSampler", "distance_transform", "coastline_stats", "coastline_metrics", "label_components", "component_stats", "remove_small_regions", "DataParallel", "GradBucketer", "FusedAdam", "UNet", "CrossEntropyArgmaxLoss"]
+           "metrics_from_counts", "METRIC_KEYS", "View", "preprocess", "resize", "enhance_image", "coastline_mask", "predict_tiled", "PatchSampler", "distance_transform", "coastline_stats", "coastline_metrics", "label_components", "component_stats", "remove_small_regions", "find_contours", "DataParallel", "GradBucketer", "FusedAdam", "UNet", "CrossEntropyArgmaxLoss"]

@@ -290,7 +290,7 @@ def enhance_image(img: torch.Tensor, enhance_water: bool = True, return_percenti
 
 def coastline_mask(mask: torch.Tensor, ksize: int = 5) -> torch.Tensor:
     """predict_coastline.py:595-602 on the GPU: cv2.dilate(mask, ellipse(ksize)) - mask for a uint8 CUDA mask [H,W] or
-    [B,H,W].  The contour tracing that follows in the reference stays on the host."""
+    [B,H,W].  The contour tracing that follows in the reference is rbunet.find_contours."""
     if not mask.is_cuda or mask.dtype != torch.uint8 or mask.dim() not in (2, 3):
         raise RuntimeError("rbunet.coastline_mask expects a uint8 CUDA tensor [H,W] or [B,H,W] (no CPU fallback)")
     single = mask.dim() == 2

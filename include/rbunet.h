@@ -60,8 +60,9 @@ size_t rbu_enhance_workspace_bytes(int B, int C, int bits);
 int rbu_enhance_image(const void* img, int bits, int B, int H, int W, int C, int enhance_water, uint8_t* out,
                       double* percentiles_out, void* workspace, size_t workspace_bytes, void* stream);
 /* rbu_coastline_mask: predict_coastline.py:595-602 -- cv2.dilate(mask, getStructuringElement(MORPH_ELLIPSE, (k,k)),
- * iterations=1) - mask on uint8 [B,H,W] masks (any values; uint8 arithmetic), 1 <= ksize <= 64.  Contour tracing
- * (cv2.findContours / approxPolyDP, :605-616) stays on the host. */
+ * iterations=1) - mask on uint8 [B,H,W] masks (any values; uint8 arithmetic), 1 <= ksize <= 64.  The contours of the
+ * band (cv2.findContours, :605-616) come from rbu_trace_contours / rbu_write_contours below; cv2.approxPolyDP stays on the
+ * host. */
 int rbu_coastline_mask(const uint8_t* mask, int B, int H, int W, int ksize, uint8_t* out, void* stream);
 /* Resizing of uint8 images (C = 3, RGB) and masks (C = 1), bit-exact with the library calls of the reference.  One
  * launch per call for a batch of sources of different sizes, all resized to oh x ow.  srcs_device: DEVICE array of B
@@ -474,6 +475,36 @@ size_t rbu_remove_small_regions_workspace_bytes(int B, int H, int W);
 int rbu_remove_small_regions(const void* mask, int kind, float threshold, int B, int H, int W, int connectivity,
                              int min_water, int min_land, uint8_t* out_u8, void* workspace, size_t workspace_bytes,
                              void* stream);
+
+/* ------------------------------------------------------------------ outer contours of water masks
+ * cv2.findContours(mask, RETR_EXTERNAL, CHAIN_APPROX_NONE | CHAIN_APPROX_SIMPLE) bit for bit, in cv2's order: the
+ * coastline polygons of predict_coastline.py:605-616 without copying the mask to the host.  mask and kind as for
+ * rbu_label_components.
+ *  - Foreground components are 8-connected; the image is framed by background.  A component is traced iff the
+ *    4-connected background component (frame included) holding the pixel above its raster-first pixel p0 touches the
+ *    frame (islands in lakes are not traced).  Contours come in decreasing raster order of p0.
+ *  - Chain codes 0 = (+1,0), 1 = (+1,-1), 2 = (0,-1) ... 7 = (+1,+1), y down.  From p0 the first foreground neighbour i1
+ *    among codes 4, 3, 2, 1, 0, 7, 6, 5 (none: the contour is the single point p0).  A state (p, c) has c pointing at
+ *    the previous pixel; its successor scans c+1, c+2, ... (mod 8) around p for the first foreground neighbour q at code
+ *    d and is (q, (d+4) mod 8).  The contour is the cycle of states from (p0, code of i1), one point per state.
+ *  - approx RBU_APPROX_NONE keeps every point, RBU_APPROX_SIMPLE the points where the chain code changes (cv2's values).
+ * Two calls, because the output is sized on the host:
+ * rbu_trace_contours: counts_out int64 [B][2] = (contours, points) per image; the workspace
+ * (rbu_contours_workspace_bytes(B, H, W) bytes, 16-byte aligned; about 46 per pixel) keeps the traced states.  Fixed
+ * launch count for given B, H, W: two union-find labellings (foreground at 8, background at 4; three launches each),
+ * frame flags, neighbour masks, state scan, state bases, links, ceil(log2(8/3 (H*W + 2H + 2W + 4))) rounds of pointer
+ * jumping, contour counts, contour scan.
+ * rbu_write_contours (after rbu_trace_contours on the same stream and workspace; repeatable): image b's n_b + 1 offsets go to
+ * offsets_out[contour_offsets[b] ...] (int64, relative to the image's first point; the last is N_b) and its N_b (x, y)
+ * int32 points to points_out[2 * point_offsets[b] ...]; contour_offsets, point_offsets: DEVICE int64 [B].  Two
+ * launches.  Integer atomics only (in the labelling): the same bits run to run and for an image alone or in a batch. */
+#define RBU_APPROX_NONE (1)
+#define RBU_APPROX_SIMPLE (2)
+size_t rbu_contours_workspace_bytes(int B, int H, int W);
+int rbu_trace_contours(const void* mask, int kind, float threshold, int B, int H, int W, int approx, int64_t* counts_out,
+                       void* workspace, size_t workspace_bytes, void* stream);
+int rbu_write_contours(void* workspace, size_t workspace_bytes, int B, int H, int W, const int64_t* contour_offsets,
+                       const int64_t* point_offsets, int64_t* offsets_out, int32_t* points_out, void* stream);
 
 #ifdef __cplusplus
 }
