@@ -111,32 +111,15 @@ __device__ __forceinline__ bool tile_coords(const HParams& p, int tile, int rank
   return !PAIR || sp < p.sp_total;
 }
 
-// barrier / TMA / MMA primitives of the single-CTA and the CTA-pair (cta_group::2) instantiation
-// Barriers completed by tcgen05.commit or TMA complete_tx are polled with the CTA-scope wait in both instantiations (the
-// data they guard travels through the async proxy / TMEM); only the accumulator-empty barriers, which collect
-// release.cluster arrivals from the peer CTA's epilogue threads, need the cluster-scope acquire.
-template <bool PAIR> __device__ __forceinline__ void bar_wait_remote(uint64_t* b, uint32_t par) {
-  if (PAIR) ptx::mbar_wait_cluster(b, par); else ptx::mbar_wait(b, par);
-}
-template <bool PAIR> __device__ __forceinline__ void load_4d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2, int c3) {
-  if (PAIR) ptx::tma_load_4d_pair(dst, m, bar, c0, c1, c2, c3); else ptx::tma_load_4d(dst, m, bar, c0, c1, c2, c3);
-}
-template <bool PAIR> __device__ __forceinline__ void load_2d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
-  if (PAIR) ptx::tma_load_2d_pair(dst, m, bar, c0, c1); else ptx::tma_load_2d(dst, m, bar, c0, c1);
-}
-template <bool PAIR> __device__ __forceinline__ void mma(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-  if (PAIR) ptx::umma_bf16_pair(d, a, b, idesc, acc); else ptx::umma_bf16(d, a, b, idesc, acc);
-}
-template <bool PAIR> __device__ __forceinline__ void commit_s(uint32_t bar) {
-  if (PAIR) ptx::umma_commit_pair(bar, 3); else ptx::umma_commit_s(bar);
-}
-
 // PAIR = true: the kernel runs as thread-block clusters of two CTAs (cta_group::2).  Each CTA owns its own spatial tile
 // (halo in its own shared memory = 128 + 128 of the M = 256 rows of every MMA) and HALF of the weight tile (block_n / 2
 // output channels: the B operand of a pair MMA is split along N between the two CTAs' shared memory), so the weight
 // bytes per SM -- L2 -> SM traffic and shared-memory operand fetch -- halve.  Only the leader (cluster rank 0) issues
 // MMAs; its commits are multicast to both CTAs' empty / accumulator-full barriers, both CTAs' TMA loads count on the
 // leader's full barriers, and both epilogues arrive on the leader's accumulator-empty barriers.
+// Barriers completed by tcgen05.commit or TMA complete_tx are polled with the CTA-scope wait in both instantiations (the
+// data they guard travels through the async proxy / TMEM); only the accumulator-empty barriers, which collect
+// release.cluster arrivals from the peer CTA's epilogue threads, need the cluster-scope acquire (ptx::bar_wait_remote).
 template <bool PAIR>
 __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CUtensorMap& tmB0, const CUtensorMap& tmA1,
                                                const CUtensorMap& tmB1, const CUtensorMap& tmY, const HParams& p) {
@@ -226,9 +209,9 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
         if (rank == 0) ptx::mbar_arrive_expect_tx(&fullA[s], txm * (halo ? A_HALO_TX : A_PLAIN_BYTES));
         const CUtensorMap* mA = ia.seg ? &tmA1 : &tmA0;
         if (halo)
-          load_4d<PAIR>(smA + s * A_HALO_BYTES, mA, &fullA[s], ia.kc * BLOCK_K, w0 - 1, h0 - 1, n);
+          ptx::load_4d<PAIR>(smA + s * A_HALO_BYTES, mA, &fullA[s], ia.kc * BLOCK_K, w0 - 1, h0 - 1, n);
         else
-          load_4d<PAIR>(smA + s * A_HALO_BYTES, mA, &fullA[s], ia.kc * BLOCK_K, w0, h0, n);
+          ptx::load_4d<PAIR>(smA + s * A_HALO_BYTES, mA, &fullA[s], ia.kc * BLOCK_K, w0, h0, n);
         ia.next(p);
       };
       if (p.resident) {
@@ -237,7 +220,7 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
         if (rank == 0) ptx::mbar_arrive_expect_tx(&fullB[0], txm * (uint32_t)(slabs * 9 * b_bytes));
         for (int kc = 0; kc < slabs; ++kc)
           for (int tap = 0; tap < 9; ++tap)
-            load_2d<PAIR>(smB + (kc * 9 + tap) * b_bytes, &tmB0, &fullB[0], tap * p.C[0] + kc * BLOCK_K, rank * bn_cta);
+            ptx::load_2d<PAIR>(smB + (kc * 9 + tap) * b_bytes, &tmB0, &fullB[0], tap * p.C[0] + kc * BLOCK_K, rank * bn_cta);
         while (ia.valid) issue_a();
       }
       if (!p.resident && ia.valid) issue_a();
@@ -255,8 +238,8 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
           ptx::mbar_wait_backoff(&emptyB[s], ph ^ 1);
           if (rank == 0) ptx::mbar_arrive_expect_tx(&fullB[s], txm * (uint32_t)(b_bytes * tps));
           for (int j = 0; j < tps; ++j)
-            load_2d<PAIR>(smB + s * bs_bytes + j * b_bytes, mB, &fullB[s], (tap0 + j) * p.C[ib.seg] + ib.kc * BLOCK_K,
-                          nb * p.block_n + rank * bn_cta);
+            ptx::load_2d<PAIR>(smB + s * bs_bytes + j * b_bytes, mB, &fullB[s], (tap0 + j) * p.C[ib.seg] + ib.kc * BLOCK_K,
+                               nb * p.block_n + rank * bn_cta);
           if (tap0 <= look && look < tap0 + tps && ia.valid) issue_a();
         }
         ib.next(p);
@@ -283,8 +266,8 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
       // half-tiles 2t (left) and 2t+1 (right) of this CTA's t-th tile: accumulator slots and their use counts
       const int sl = (2 * t) & p.slot_mask, sr = (2 * t + 1) & p.slot_mask;
       const uint32_t use_par = (uint32_t)((2 * t) >> p.slot_shift) & 1u;
-      bar_wait_remote<PAIR>(&tempty[sl], use_par ^ 1);
-      bar_wait_remote<PAIR>(&tempty[sr], use_par ^ 1);
+      ptx::bar_wait_remote<PAIR>(&tempty[sl], use_par ^ 1);
+      ptx::bar_wait_remote<PAIR>(&tempty[sr], use_par ^ 1);
       ptx::tc_fence_after();
       const uint32_t d_l = tmem_base + (uint32_t)(sl * p.block_n), d_r = tmem_base + (uint32_t)(sr * p.block_n);
       const int cur_tile = it.tile;
@@ -318,8 +301,8 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
                   const uint64_t bd = ptx::pack_desc(b_lo + (dy * 3 + dx) * b_step + 2 * k, b_hi);
                   const uint32_t al = a_lo0 + dy * ROW_OFF + dx * 8 + 2 * k;
                   const uint32_t acc = (dy | dx | k) ? 1u : accumulate;
-                  mma<PAIR>(d_l, ptx::pack_desc(al, a_hi), bd, idesc, acc);
-                  mma<PAIR>(d_r, ptx::pack_desc(al + HALF_OFF, a_hi), bd, idesc, acc);
+                  ptx::mma<PAIR>(d_l, ptx::pack_desc(al, a_hi), bd, idesc, acc);
+                  ptx::mma<PAIR>(d_r, ptx::pack_desc(al + HALF_OFF, a_hi), bd, idesc, acc);
                 }
           }
           accumulate = 1;
@@ -338,11 +321,11 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
                 for (int k = 0; k < 4; ++k) {
                   const uint64_t bd = ptx::pack_desc(b_lo + dx * b_step + 2 * k, b_hi);
                   const uint32_t acc = (dx | k) ? 1u : accumulate;
-                  mma<PAIR>(d_l, ptx::pack_desc(a_row + dx * 8 + 2 * k, a_hi), bd, idesc, acc);
-                  mma<PAIR>(d_r, ptx::pack_desc(a_row + HALF_OFF + dx * 8 + 2 * k, a_hi), bd, idesc, acc);
+                  ptx::mma<PAIR>(d_l, ptx::pack_desc(a_row + dx * 8 + 2 * k, a_hi), bd, idesc, acc);
+                  ptx::mma<PAIR>(d_r, ptx::pack_desc(a_row + HALF_OFF + dx * 8 + 2 * k, a_hi), bd, idesc, acc);
                 }
               }
-              commit_s<PAIR>(emptyB_s + sb * 8);
+              ptx::commit_s<PAIR>(emptyB_s + sb * 8);
             }
             accumulate = 1;
             __syncwarp();
@@ -364,12 +347,12 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
               for (int k = 0; k < 4; ++k) {
                 if (k < ksteps) {
                   const uint64_t bd = ptx::pack_desc(b_lo + 2 * k, b_hi);
-                  mma<PAIR>(d_l, ptx::pack_desc(a_lo + 2 * k, a_hi), bd, idesc, accumulate);
-                  mma<PAIR>(d_r, ptx::pack_desc(a_lo + HALF_OFF + 2 * k, a_hi), bd, idesc, accumulate);
+                  ptx::mma<PAIR>(d_l, ptx::pack_desc(a_lo + 2 * k, a_hi), bd, idesc, accumulate);
+                  ptx::mma<PAIR>(d_r, ptx::pack_desc(a_lo + HALF_OFF + 2 * k, a_hi), bd, idesc, accumulate);
                   accumulate = 1;
                 }
               }
-              if (j == tps - 1) commit_s<PAIR>(emptyB_s + sb * 8);
+              if (j == tps - 1) ptx::commit_s<PAIR>(emptyB_s + sb * 8);
             }
             accumulate = 1;
             __syncwarp();
@@ -380,14 +363,14 @@ __device__ __forceinline__ void conv_halo_body(const CUtensorMap& tmA0, const CU
             if (++dx == 3) { dx = 0; a_row += ROW_OFF; a_lo = a_row; } else { a_lo += 128 >> 4; }
           }
         }
-        if (ptx::elect_one()) commit_s<PAIR>(emptyA_s + sa * 8);
+        if (ptx::elect_one()) ptx::commit_s<PAIR>(emptyA_s + sa * 8);
         __syncwarp();
         if (++sa == p.a_stages) { sa = 0; pha ^= 1; }
         it.next(p);
       }
       if (ptx::elect_one()) {
-        commit_s<PAIR>(ptx::smem_u32(&tfull[sl]));
-        commit_s<PAIR>(ptx::smem_u32(&tfull[sr]));
+        ptx::commit_s<PAIR>(ptx::smem_u32(&tfull[sl]));
+        ptx::commit_s<PAIR>(ptx::smem_u32(&tfull[sr]));
       }
       __syncwarp();
       ++t;

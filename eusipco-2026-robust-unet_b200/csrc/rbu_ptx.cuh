@@ -332,6 +332,25 @@ __device__ __forceinline__ uint32_t desc_hi_sw32(uint32_t sbo_bytes) {
   return ((sbo_bytes >> 4) & 0x3FFFu) | (1u << 14) | (6u << 29);
 }
 
+// The same step in a kernel instantiated for one CTA (PAIR = false) or for a CTA pair (PAIR = true, cta_group::2):
+// barrier wait (the pair's with cluster-scope acquire), TMA load (the pair's counted on the leader's barrier), MMA issue,
+// and commit (the pair's multicast to the barrier at the same offset in both CTAs).
+template <bool PAIR> __device__ __forceinline__ void bar_wait_remote(uint64_t* b, uint32_t par) {
+  if (PAIR) mbar_wait_cluster(b, par); else mbar_wait(b, par);
+}
+template <bool PAIR> __device__ __forceinline__ void load_4d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2, int c3) {
+  if (PAIR) tma_load_4d_pair(dst, m, bar, c0, c1, c2, c3); else tma_load_4d(dst, m, bar, c0, c1, c2, c3);
+}
+template <bool PAIR> __device__ __forceinline__ void load_2d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
+  if (PAIR) tma_load_2d_pair(dst, m, bar, c0, c1); else tma_load_2d(dst, m, bar, c0, c1);
+}
+template <bool PAIR> __device__ __forceinline__ void mma(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
+  if (PAIR) umma_bf16_pair(d, a, b, idesc, acc); else umma_bf16(d, a, b, idesc, acc);
+}
+template <bool PAIR> __device__ __forceinline__ void commit_s(uint32_t bar) {
+  if (PAIR) umma_commit_pair(bar, 3); else umma_commit_s(bar);
+}
+
 // ----------------------------------------------------------------------------- descriptors
 // Shared-memory matrix descriptor, SWIZZLE_128B, sm_100 version field = 1.
 //   K-major operand  (rows = M/N index, 128 B = 64 bf16 of K per row): SBO = 1024 B (8-row group), LBO unused.

@@ -297,9 +297,9 @@ def test_gpu_reference_matches_cpu_reference():
         assert torch.equal(cpu, gpu), name
 
 
-# Weight-gradient rows.  Halo kernels: wgrad_halo.cu:568-570 (3x3 dil 1, H >= 8, W >= 16), forms wgrad_halo.cu:532-539
+# Weight-gradient rows.  Halo kernels: wgrad_halo.cu:428-430 (3x3 dil 1, H >= 8, W >= 16), forms wgrad_halo.cu:394-399
 # (form 2 when Cout % 128 == 0 and Cin % 32 == 0, the pair form when also Cout % 256 == 0, else form 1); split-K from the
-# cost model wgrad_halo.cu:543-563.  Generic kernel: wgrad_gemm.cu:440-445 and :300-344 (ksplit = ceil(2 * SMs /
+# cost model wgrad_halo.cu:404-421 with the per-form tile times of form_shape, :84-91.  Generic kernel: wgrad_gemm.cu:440-445 and :300-344 (ksplit = ceil(2 * SMs /
 # items), capped by the pixel tiles).  Reduction kernel: wgrad_gemm.cu:358-367 (<64> for Cin >= 64 and ksplit <= 16, <32>
 # for Cin >= 32 and ksplit <= 64, else <16>).  The ksplit values in the comments are for 148 SMs.
 WGRAD_ROWS = [
